@@ -17,6 +17,9 @@ e2e      : the same metric through the reference-facing call bspatom_solve_batch
            the reference keeps are computed and copied, and they are gathered over NCCL to rank 0.
 --impl reference : the reference's own CPU algorithm (oracle restatement of MATRIX_SVT + LAPACK dsygv with the
            arguments of matrices.f90:248) on the box's host cores, bounded sample per step.
+--dump-outputs DIR : after the timed steps, rank 0 writes what the timed call returned in the last step as DIR/<name>.npy
+           (float64, at most 60 MB in all; outputs larger than that as a fixed, seeded sample of rows plus the row
+           indices), so that two builds can be compared output for output on identical inputs.
 """
 from __future__ import annotations
 
@@ -45,6 +48,29 @@ LABELS = {"cfg2": "cfg2 Coulomb l=0..50 N=1000 k=7 Rmax=500 all eigenpairs (%s k
 
 def label(cfg, grid):
     return LABELS[cfg] % grid if "%s" in LABELS[cfg] else LABELS[cfg]
+
+
+DUMP_BYTES = 60 * 1000 * 1000        # data of all files; .npy headers add 128 bytes each
+DUMP_SEED = 20261020
+
+
+def sample_rows(nrows: int, row_bytes: int, budget: int) -> np.ndarray:
+    """ascending indices of a fixed, seeded sample of rows that fits in `budget` bytes (every row when all fit)"""
+    m = min(nrows, budget // row_bytes)
+    if m == nrows:
+        return np.arange(nrows)
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(nrows, size=m, replace=False))
+
+
+def dump_outputs(directory: str, arrays: dict):
+    """writes each array as <directory>/<name>.npy in float64"""
+    arrays = {nm: np.ascontiguousarray(a, dtype=np.float64) for nm, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_BYTES))
+    os.makedirs(directory, exist_ok=True)
+    for nm, a in arrays.items():
+        np.save(os.path.join(directory, nm + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------
@@ -319,7 +345,12 @@ def main():
     ap.add_argument("--no-numa", action="store_true", help="do not bind host memory / CPU affinity to the GPU's NUMA node")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -402,6 +433,18 @@ def main():
     info = np.zeros(nsolve, dtype=np.int32)
     atom.batch_download(E_host, None, info)
     E_last = np.array(E_host).reshape(nsolve, NFUN)
+    if args.dump_outputs and rank == 0:
+        # what bspatom_batch_download hands a caller after the last timed step: every eigenvalue and info code, and the
+        # eigenvectors (GBs: a sample of them).  Problem i's block is nfun x nvec column-major with nvec = nfun, so
+        # row r of C_dev is eigenvector r % NFUN of problem r // NFUN.
+        C_dev = torch.empty((nsolve * NFUN, NFUN), dtype=torch.float64, device="cuda")
+        atom.batch_download_ptrs(0, C_dev.data_ptr())
+        rows = sample_rows(nsolve * NFUN, 8 * (NFUN + 1), DUMP_BYTES - E_last.nbytes - 8 * nsolve)
+        C_rows = C_dev[torch.from_numpy(rows).to(C_dev.device)].cpu().numpy()
+        del C_dev
+        torch.cuda.empty_cache()
+        dump_outputs(args.dump_outputs, {"eigenvalues": E_last, "info": info, "eigenvectors_sample": C_rows,
+                                         "eigenvectors_sample_rows": rows})
     accuracy = {"pencils_checked_on_device": nsolve, "eigenpairs_checked_on_device": ver["eigenpairs_checked"],
                 "max_scaled_residual": ver["max_scaled_residual"], "max_CtSC_minus_I": ver["max_orthonormality_defect"],
                 "spectra_strictly_ascending": ver["not_ascending"] == 0.0, "info_nonzero": int(np.count_nonzero(info)),
@@ -706,6 +749,11 @@ def bench_cfg5(args, torch, dist, bsp, world, rank, local, barrier, allmax):
     wall_res = allmax(time.perf_counter() - t0)
     sampler.stop_flag = True
     sampler.join(timeout=2)
+    if args.dump_outputs and rank == 0:
+        # D[l][i, j] = <state i of l+1| r |state j of l>; row r of D_rows is D[r // n][r % n, :]
+        D_rows = np.ascontiguousarray(D).reshape(-1, n)
+        rows = sample_rows(D_rows.shape[0], 8 * (n + 1), DUMP_BYTES)
+        dump_outputs(args.dump_outputs, {"dipole_sample": D_rows[rows], "dipole_sample_rows": rows})
     ms = allmax(ms)
     tf = flops * args.steps * world / (ms * 1e-3) / 1e12
     # e2e: host blocks in, D out
