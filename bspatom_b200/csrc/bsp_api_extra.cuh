@@ -633,8 +633,11 @@ int bspatom_batch_verify(bspatom_handle h, double *out)
     CU(cudaMemsetAsync(d_out, 0, 4 * sizeof(double), h->st));
     double checked = 0.0;
     for (auto &G : h->groups) {
+        /* with a device-side selection only the first nsel columns of a pencil were computed: check those */
+        std::vector<int> nvec(G.npencil);
+        const int *d_nvec = G.any_sel ? G.d_nvec_eff : G.d_nvec;
         int maxnv = 0;
-        for (int p = 0; p < G.npencil; ++p) maxnv = std::max(maxnv, G.nvec[p]);
+        for (int p = 0; p < G.npencil; ++p) maxnv = std::max(maxnv, nvec[p] = resident_nvec(h, G, p));
         if (maxnv == 0) continue;
         /* scratch per pencil: Y (n x maxnv) + Gram (maxnv x maxnv); chunks of <= 2 GB */
         const size_t per = ((size_t)G.n + maxnv) * maxnv;
@@ -645,15 +648,15 @@ int bspatom_batch_verify(bspatom_handle h, double *out)
         for (int p0 = 0; p0 < G.npencil; p0 += chunk) {
             const int np = std::min(chunk, G.npencil - p0);
             bsp_verify_matvec_kernel<<<dim3((G.n + 127) / 128, maxnv, np), 128, 0, h->st>>>(
-                G.n, G.B, G.nrows, G.d_fbS, G.d_fbH0, G.d_fbQ, G.d_inst, G.d_cl, G.d_nvec, G.d_coff, G.d_C, G.d_E, d_Y,
+                G.n, G.B, G.nrows, G.d_fbS, G.d_fbH0, G.d_fbQ, G.d_inst, G.d_cl, d_nvec, G.d_coff, G.d_C, G.d_E, d_Y,
                 (long long)G.n * maxnv, p0, d_out);
             CU(cudaGetLastError());
             /* Gram matrices: pencils of a group may have different nvec, so one GEMM launch per run of equal nvec */
             int q = 0;
             while (q < np) {
                 int q1 = q;
-                const int nv = G.nvec[p0 + q];
-                while (q1 + 1 < np && G.nvec[p0 + q1 + 1] == nv &&
+                const int nv = nvec[p0 + q];
+                while (q1 + 1 < np && nvec[p0 + q1 + 1] == nv &&
                        G.coff[p0 + q1 + 1] - G.coff[p0 + q1] == (long long)G.n * nv) ++q1;
                 if (nv > 0) {
                     CU(bsp_launch_dgemm_tn(h->st, nv, nv, G.n, G.d_C + G.coff[p0 + q], G.n, d_Y + (size_t)q * G.n * maxnv, G.n,
@@ -663,11 +666,11 @@ int bspatom_batch_verify(bspatom_handle h, double *out)
                 q = q1 + 1;
             }
             bsp_verify_gram_kernel<<<dim3((std::max(maxnv, G.n) + 127) / 128, maxnv, np), 128, 0, h->st>>>(
-                G.n, G.d_nvec, d_G, (long long)maxnv * maxnv, maxnv, G.d_E, p0, d_out);
+                G.n, d_nvec, d_G, (long long)maxnv * maxnv, maxnv, G.d_E, p0, d_out);
             CU(cudaGetLastError());
             h->launches += 3;
         }
-        for (int p = 0; p < G.npencil; ++p) checked += G.nvec[p];
+        for (int p = 0; p < G.npencil; ++p) checked += nvec[p];
         CU(cudaStreamSynchronize(h->st));
         dev_free(h, d_Y, (size_t)chunk * G.n * maxnv);
         dev_free(h, d_G, (size_t)chunk * maxnv * maxnv);

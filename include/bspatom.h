@@ -159,7 +159,8 @@ int bspatom_get_selection(bspatom_handle h, int *nsel);
 
 /* device-side check of the resident batch (after bspatom_batch_run): out[0] = max scaled residual
  * |H_l c - E S c|_inf / max(1,|E|) over EVERY eigenpair, out[1] = max |C^T S C - I| over every pencil,
- * out[2] = 0 when every spectrum is strictly ascending, out[3] = eigenpairs checked.  What the host would
+ * out[2] = 0 when every spectrum is strictly ascending, out[3] = eigenpairs checked (with sel_mode = 1: the
+ * selected ones, bspatom_get_selection, since only those eigenvectors were computed).  What the host would
  * otherwise verify after gathering Hij (matrices.f90:248) -- without moving the eigenvectors.           */
 int bspatom_batch_verify(bspatom_handle h, double *out4);
 
