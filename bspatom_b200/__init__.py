@@ -5,7 +5,7 @@ Only what the path needs lives here: ``csrc/`` (CUDA kernels + the C-ABI), ``_li
 binding), ``host`` (mirror of the reference driver's interface), ``parallel`` (sharding of the
 (instance, l) list over one-process-per-GPU ranks and the single eigenpair gather)."""
 from ._lib import BspAtomError, LIB_PATH, load  # noqa: F401
-from .host import (BspAtom, BspAtomMulti, BspAtomPipeline, BspInputs, Problem, Selection, dsygv, parse_namelists,  # noqa: F401
+from .host import (BspAtom, BspAtomMulti, BspAtomPipeline, BspInputs, Problem, Selection, dsbgv, dsygv, parse_namelists,  # noqa: F401
                    POT_COULOMB, POT_ROGERS, POT_SIMONS_FUES, POT_TABLE, POT_TIETZ, POT_YUKAWA)
 from .parallel import gather_eigenpairs, gather_eigenpairs_device, shard_items  # noqa: F401
 

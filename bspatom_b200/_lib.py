@@ -22,6 +22,7 @@ EXPORTS = [
     "bspatom_batch_download", "bspatom_get_selection", "bspatom_batch_verify", "bspatom_dsygv_", "bspatom_dipole", "bspatom_dipole_chain", "bspatom_dipole_chain_resident",
     "bspatom_create_multi", "bspatom_destroy_multi", "bspatom_last_error_multi", "bspatom_set_option_multi", "bspatom_solve_batch_multi",
     "bspatom_trans_amp_hermitian", "bspatom_assemble_zaij", "bspatom_wavefunction", "bspatom_wavefunction_resident", "bspatom_get_stats",
+    "bspatom_band_upload", "bspatom_solve_band_batch", "bspatom_dsbgv_",
 ]
 
 
@@ -36,6 +37,15 @@ class BspProblem(C.Structure):
         ("l", C.c_int), ("ul_extra", C.c_double), ("nvec", C.c_int),
         ("sel_mode", C.c_int), ("sel_extra", C.c_int), ("sel_group", C.c_int),
         ("sel_ecut_a", C.c_double), ("sel_ecut_b", C.c_double),
+    ]
+
+
+class BspBandPencil(C.Structure):
+    """struct bsp_band_pencil of include/bspatom.h"""
+
+    _fields_ = [
+        ("n", C.c_int), ("ka", C.c_int), ("kb", C.c_int), ("uplo", C.c_char),
+        ("AB", _dp), ("ldab", C.c_int), ("BB", _dp), ("ldbb", C.c_int), ("nvec", C.c_int),
     ]
 
 
@@ -94,6 +104,11 @@ def load():
     L.bspatom_wavefunction_resident.argtypes = [H, C.c_int, C.c_int, C.c_int, C.c_double, C.c_double, C.c_int,
                                                 C.c_void_p, C.c_void_p]
     L.bspatom_get_stats.argtypes = [H, _dp, C.c_int]
+    L.bspatom_band_upload.argtypes = [H, C.c_int, C.POINTER(BspBandPencil)]
+    L.bspatom_solve_band_batch.argtypes = [H, C.c_int, C.POINTER(BspBandPencil), C.c_void_p, C.c_void_p, C.c_void_p]
+    L.bspatom_dsbgv_.argtypes = [C.c_char_p, C.c_char_p, _ip, _ip, _ip, C.c_void_p, _ip, C.c_void_p, _ip, C.c_void_p,
+                                 C.c_void_p, _ip, C.c_void_p, _ip]
+    L.bspatom_dsbgv_.restype = None
     _lib = L
     return L
 

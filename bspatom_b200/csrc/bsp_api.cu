@@ -15,6 +15,7 @@
 #include <stdlib.h>
 #include <string.h>
 #include <algorithm>
+#include <cmath>
 #include <chrono>
 #include <mutex>
 #include <map>
@@ -61,6 +62,7 @@ struct Group {
     int k = 0, B = 0, n = 0, nkp = 0, ka = 0, npad = 0, nrows = 0, xrows = 0, ldw = 0, FS = 0;
     int ninst = 0, npencil = 0;
     bool any_vtab = false;
+    bool band = false; /* ingested from caller-supplied bands (bspatom_band_upload): no knots, nothing to assemble */
     int budget_pencils = 0; /* pencils whose workspaces fit the memory budget (decided on the first run) */
     std::vector<int> prob_index; /* pencil -> caller's problem index */
     std::vector<int> inst, nvec;
@@ -104,6 +106,10 @@ struct bspatom_handle_s {
     std::vector<long long> e_off, c_off; /* per caller problem: offsets in E and C */
     std::vector<int> p_n, p_nvec;
     bool uploaded = false, ran = false;
+    bool band = false;                      /* the batch came from bspatom_band_upload */
+    std::vector<std::pair<int, int>> outside; /* (problem, info) of band pencils in no group: n = 0, or B not PD */
+    double *h_stage = nullptr;              /* pinned staging of bspatom_band_upload, h_stage_cap doubles */
+    size_t h_stage_cap = 0;
     Workspace ws;
     /* freed device buffers by byte size: a sweep re-submits batches of identical shape, and
      * cudaMalloc/cudaFree of the multi-GB result buffers costs tens of ms per call */
@@ -217,6 +223,8 @@ void free_batch(bspatom_handle h)
     for (auto &g : h->groups) free_group(h, g);
     h->groups.clear();
     h->uploaded = h->ran = false;
+    h->band = false;
+    h->outside.clear();
 }
 
 /* Gauss-Legendre nodes/weights on [-1,1] by Newton iteration on P_n with the
@@ -664,6 +672,35 @@ int upload_group_instances(bspatom_handle h, Group &G, const std::vector<const b
     return 0;
 }
 
+/* per-pencil tables of a group (instance, nvec, c_l, C offset, selection rule) and its result buffers */
+int upload_group_pencils(bspatom_handle h, Group &G)
+{
+    int rc;
+    if ((rc = dev_alloc(h, &G.d_inst, G.npencil))) return rc;
+    if ((rc = dev_alloc(h, &G.d_nvec, G.npencil))) return rc;
+    if ((rc = dev_alloc(h, &G.d_cl, G.npencil))) return rc;
+    if ((rc = dev_alloc(h, &G.d_coff, G.npencil))) return rc;
+    if ((rc = dev_alloc(h, &G.d_bad, G.npencil))) return rc;
+    if ((rc = dev_alloc(h, &G.d_E, (size_t)G.npencil * G.n))) return rc;
+    if ((rc = dev_alloc(h, &G.d_C, (size_t)G.c_elems))) return rc;
+    CU(cudaMemcpyAsync(G.d_inst, G.inst.data(), sizeof(int) * G.npencil, cudaMemcpyHostToDevice, h->st));
+    CU(cudaMemcpyAsync(G.d_nvec, G.nvec.data(), sizeof(int) * G.npencil, cudaMemcpyHostToDevice, h->st));
+    std::vector<int> nvec_br(G.nvec);
+    if (G.any_sel) {
+        for (int p = 0; p < G.npencil; ++p) if (G.sel[p].mode) nvec_br[p] = 0;
+        if ((rc = dev_alloc(h, &G.d_sel, G.npencil))) return rc;
+        if ((rc = dev_alloc(h, &G.d_nvec_br, G.npencil))) return rc;
+        if ((rc = dev_alloc(h, &G.d_nvec_eff, G.npencil))) return rc;
+        CU(cudaMemcpyAsync(G.d_sel, G.sel.data(), sizeof(BspSelect) * G.npencil, cudaMemcpyHostToDevice, h->st));
+        CU(cudaMemcpyAsync(G.d_nvec_br, nvec_br.data(), sizeof(int) * G.npencil, cudaMemcpyHostToDevice, h->st));
+        CU(cudaMemcpyAsync(G.d_nvec_eff, G.nvec.data(), sizeof(int) * G.npencil, cudaMemcpyHostToDevice, h->st));
+    }
+    CU(cudaMemcpyAsync(G.d_cl, G.cl.data(), sizeof(double) * G.npencil, cudaMemcpyHostToDevice, h->st));
+    CU(cudaMemcpyAsync(G.d_coff, G.coff.data(), sizeof(long long) * G.npencil, cudaMemcpyHostToDevice, h->st));
+    CU(cudaStreamSynchronize(h->st));
+    return 0;
+}
+
 bspatom_handle new_context(int device_id)
 {
     bspatom_handle h = new bspatom_handle_s();
@@ -689,6 +726,7 @@ void free_context(bspatom_handle h)
     for (auto e : h->ev_pool) cudaEventDestroy(e);
     if (h->h_counter) cudaFreeHost(h->h_counter);
     if (h->h_sel) cudaFreeHost(h->h_sel);
+    if (h->h_stage) cudaFreeHost(h->h_stage);
     for (auto e : h->chunk_done) cudaEventDestroy(e);
     if (h->st_copy) cudaStreamDestroy(h->st_copy);
     if (h->st) cudaStreamDestroy(h->st);
@@ -880,29 +918,8 @@ int bspatom_batch_upload(bspatom_handle h, int nprob, const bsp_problem *probs)
         if ((rc = dev_alloc(h, &G.d_fbS, per_mat * G.ninst))) return rc;
         if ((rc = dev_alloc(h, &G.d_fbH0, per_mat * G.ninst))) return rc;
         if ((rc = dev_alloc(h, &G.d_fbQ, per_mat * G.ninst))) return rc;
-        if ((rc = dev_alloc(h, &G.d_inst, G.npencil))) return rc;
-        if ((rc = dev_alloc(h, &G.d_nvec, G.npencil))) return rc;
-        if ((rc = dev_alloc(h, &G.d_cl, G.npencil))) return rc;
-        if ((rc = dev_alloc(h, &G.d_coff, G.npencil))) return rc;
         if ((rc = dev_alloc(h, &G.d_pdinfo, G.ninst))) return rc;
-        if ((rc = dev_alloc(h, &G.d_bad, G.npencil))) return rc;
-        if ((rc = dev_alloc(h, &G.d_E, (size_t)G.npencil * G.n))) return rc;
-        if ((rc = dev_alloc(h, &G.d_C, (size_t)G.c_elems))) return rc;
-        CU(cudaMemcpyAsync(G.d_inst, G.inst.data(), sizeof(int) * G.npencil, cudaMemcpyHostToDevice, h->st));
-        CU(cudaMemcpyAsync(G.d_nvec, G.nvec.data(), sizeof(int) * G.npencil, cudaMemcpyHostToDevice, h->st));
-        std::vector<int> nvec_br(G.nvec);
-        if (G.any_sel) {
-            for (int p = 0; p < G.npencil; ++p) if (G.sel[p].mode) nvec_br[p] = 0;
-            if ((rc = dev_alloc(h, &G.d_sel, G.npencil))) return rc;
-            if ((rc = dev_alloc(h, &G.d_nvec_br, G.npencil))) return rc;
-            if ((rc = dev_alloc(h, &G.d_nvec_eff, G.npencil))) return rc;
-            CU(cudaMemcpyAsync(G.d_sel, G.sel.data(), sizeof(BspSelect) * G.npencil, cudaMemcpyHostToDevice, h->st));
-            CU(cudaMemcpyAsync(G.d_nvec_br, nvec_br.data(), sizeof(int) * G.npencil, cudaMemcpyHostToDevice, h->st));
-            CU(cudaMemcpyAsync(G.d_nvec_eff, G.nvec.data(), sizeof(int) * G.npencil, cudaMemcpyHostToDevice, h->st));
-        }
-        CU(cudaMemcpyAsync(G.d_cl, G.cl.data(), sizeof(double) * G.npencil, cudaMemcpyHostToDevice, h->st));
-        CU(cudaMemcpyAsync(G.d_coff, G.coff.data(), sizeof(long long) * G.npencil, cudaMemcpyHostToDevice, h->st));
-        CU(cudaStreamSynchronize(h->st));
+        if ((rc = upload_group_pencils(h, G))) return rc;
     }
     {
         size_t need = 0;
@@ -1113,12 +1130,12 @@ int run_internal(bspatom_handle h, double *E_out, double *C_out)
         const BspSchedule sch = values_only ? sch_val : sch_vec;
         /* ---- assembly, once per instance ---- */
         CU(cudaEventRecord(e1, h->st));
-        BspAsmArgs a;
-        memset(&a, 0, sizeof a);
-        a.n = G.n; a.nkp = G.nkp; a.ka = G.ka; a.nrows = G.nrows; a.ninst = G.ninst; a.want_pi = 0;
-        a.rt = G.d_rt; a.xgwg = G.d_xgwg; a.par = G.d_par; a.vtab = G.d_vtab;
-        a.fb[BSP_MAT_S] = G.d_fbS; a.fb[BSP_MAT_H0] = G.d_fbH0; a.fb[BSP_MAT_Q] = G.d_fbQ;
-        {
+        if (!G.band) {   /* a band group's rows were written by bspatom_band_upload */
+            BspAsmArgs a;
+            memset(&a, 0, sizeof a);
+            a.n = G.n; a.nkp = G.nkp; a.ka = G.ka; a.nrows = G.nrows; a.ninst = G.ninst; a.want_pi = 0;
+            a.rt = G.d_rt; a.xgwg = G.d_xgwg; a.par = G.d_par; a.vtab = G.d_vtab;
+            a.fb[BSP_MAT_S] = G.d_fbS; a.fb[BSP_MAT_H0] = G.d_fbH0; a.fb[BSP_MAT_Q] = G.d_fbQ;
             const int s = timed_begin(h, 3);
             rc = launch_assembly(h, G.k, a);
             timed_end(h, s);
@@ -1417,6 +1434,8 @@ int bspatom_batch_download(bspatom_handle h, double *E, double *C, int *info)
     if (rc) return rc;
     if (!h->ran) { h->err = "batch_download before batch_run"; return BSPATOM_ESTATE; }
     size_t mail_off = BSP_MAIL_REPORT_INTS;
+    if (info)
+        for (auto &o : h->outside) info[o.first] = o.second;
     for (auto &G : h->groups) {
         G.pdinfo.resize(G.ninst);
         G.bad.resize(G.npencil);
@@ -1467,28 +1486,221 @@ int bspatom_get_selection(bspatom_handle h, int *nsel)
     if (rc) return rc;
     if (!nsel) return -2;
     if (!h->ran) { h->err = "get_selection before a run"; return BSPATOM_ESTATE; }
+    for (auto &o : h->outside) nsel[o.first] = 0;
     for (auto &G : h->groups)
         for (int p = 0; p < G.npencil; ++p)
             nsel[G.prob_index[p]] = G.any_sel ? std::min(h->h_sel[G.sel_off + p], G.nvec[p]) : G.nvec[p];
     return 0;
 }
 
-int bspatom_solve_batch(bspatom_handle h, int nprob, const bsp_problem *probs, double *E, double *C, int *info)
+} /* extern "C" */
+
+namespace {
+
+/* run + download of an uploaded batch (upload began at host clock t0) */
+int run_and_download(bspatom_handle h, double *E, double *C, int *info, double t0)
 {
-    auto now = [] { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
-    const double t0 = now();
-    int rc = bspatom_batch_upload(h, nprob, probs);
-    if (rc) return rc;
-    const double t1 = now();
+    const double t1 = host_ms();
     /* pinned (cudaHostAlloc / cudaHostRegister / bspatom_alloc_host) output buffers are filled chunk by
      * chunk while the next chunk computes; pageable ones after the run */
     const bool pe = is_pinned(E), pc = is_pinned(C);
-    if ((rc = run_internal(h, pe ? E : nullptr, pc ? C : nullptr))) return rc;
-    const double t2 = now();
+    int rc = run_internal(h, pe ? E : nullptr, pc ? C : nullptr);
+    if (rc) return rc;
+    const double t2 = host_ms();
     rc = bspatom_batch_download(h, pe ? nullptr : E, pc ? nullptr : C, info);
-    const double t3 = now();
+    const double t3 = host_ms();
     h->stats[16] = t1 - t0; h->stats[17] = t2 - t1; h->stats[18] = t3 - t2;   /* host wall ms: upload, run(+overlapped copies), download */
     return rc;
+}
+
+bool is_upper(char uplo) { return uplo == 'U' || uplo == 'u'; }
+
+/* every entry of the stored triangle of a symmetric band in LAPACK storage (leading dimension ld) is finite */
+bool band_finite(const double *M, int ld, int k, int n, bool upper)
+{
+    for (int j = 0; j < n; ++j) {
+        const int r0 = upper ? std::max(0, k - j) : 0, r1 = upper ? k : std::min(k, n - 1 - j);
+        for (int r = r0; r <= r1; ++r)
+            if (!std::isfinite(M[(size_t)j * ld + r])) return false;
+    }
+    return true;
+}
+
+/* the stored triangle of a band -> packed storage with leading dimension k+1 (entries outside the matrix become 0) */
+void band_pack(double *dst, const double *M, int ld, int k, int n, bool upper)
+{
+    for (int j = 0; j < n; ++j) {
+        const int r0 = upper ? std::max(0, k - j) : 0, r1 = upper ? k : std::min(k, n - 1 - j);
+        for (int r = 0; r <= k; ++r) dst[(size_t)j * (k + 1) + r] = (r >= r0 && r <= r1) ? M[(size_t)j * ld + r] : 0.0;
+    }
+}
+
+/* 0, -3 (malformed; *why says how) or BSPATOM_EUNSUPPORTED */
+int validate_band(const bsp_band_pencil &q, const char *&why)
+{
+    why = "";
+    if (q.n < 0) { why = "n < 0"; return -3; }
+    if (q.ka < 0 || q.kb < 0) { why = "negative half bandwidth"; return -3; }
+    if (q.ka > BSP_KMAX - 1 || q.kb > BSP_KMAX - 1) { why = "half bandwidth above 9"; return BSPATOM_EUNSUPPORTED; }
+    if (!is_upper(q.uplo) && q.uplo != 'L' && q.uplo != 'l') { why = "uplo is neither 'U' nor 'L'"; return -3; }
+    if (q.ldab < q.ka + 1) { why = "ldab < ka + 1"; return -3; }
+    if (q.ldbb < q.kb + 1) { why = "ldbb < kb + 1"; return -3; }
+    if (q.n > 0 && (!q.AB || !q.BB)) { why = "AB or BB is NULL"; return -3; }
+    if (q.nvec < 0 || q.nvec > q.n) { why = "nvec outside 0..n"; return -3; }
+    if (q.n > 0 && !band_finite(q.AB, q.ldab, q.ka, q.n, is_upper(q.uplo))) { why = "NaN or Inf in the stored band of AB"; return -3; }
+    if (q.n > 0 && !band_finite(q.BB, q.ldbb, q.kb, q.n, is_upper(q.uplo))) { why = "NaN or Inf in the stored band of BB"; return -3; }
+    return 0;
+}
+
+template <class T>
+size_t doubles_for(size_t count) { return (count * sizeof(T) + sizeof(double) - 1) / sizeof(double); }
+
+} // namespace
+
+extern "C" {
+
+int bspatom_solve_batch(bspatom_handle h, int nprob, const bsp_problem *probs, double *E, double *C, int *info)
+{
+    const double t0 = host_ms();
+    int rc = bspatom_batch_upload(h, nprob, probs);
+    if (rc) return rc;
+    return run_and_download(h, E, C, info, t0);
+}
+
+/* Caller-supplied bands.  The host checks every pencil, then packs all bands and their descriptors into one pinned
+ * staging buffer that one copy takes to the device; per (n, B) group one ingest launch writes the full-band rows of
+ * S, H0 and Q and one launch checks S for positive definiteness.  Pencils whose S fails are dropped from their
+ * group before the per-pencil tables are built, so the solver never sees them. */
+int bspatom_band_upload(bspatom_handle h, int nprob, const bsp_band_pencil *pens)
+{
+    int rc = check_device(h);
+    if (rc) return rc;
+    if (nprob < 0) return -2;
+    if (nprob > 0 && !pens) return -3;
+    for (int i = 0; i < nprob; ++i) {   /* before any device work: a rejected batch leaves the handle as it was */
+        const char *why = "";
+        if ((rc = validate_band(pens[i], why))) { h->err = "bsp_band_pencil at index " + std::to_string(i) + ": " + why; return rc; }
+    }
+    free_batch(h);
+    h->band = true;
+    h->nprob = nprob;
+    h->e_off.assign(nprob + 1, 0);
+    h->c_off.assign(nprob + 1, 0);
+    h->p_n.assign(nprob, 0);
+    h->p_nvec.assign(nprob, 0);
+    std::map<std::pair<int, int>, int> gid;
+    std::vector<std::vector<int>> members;
+    size_t ndesc = 0, nband = 0;
+    for (int i = 0; i < nprob; ++i) {
+        const bsp_band_pencil &q = pens[i];
+        h->p_n[i] = q.n;
+        h->p_nvec[i] = q.nvec;
+        h->e_off[i + 1] = h->e_off[i] + q.n;
+        h->c_off[i + 1] = h->c_off[i] + (long long)q.n * q.nvec;
+        if (q.n == 0) { h->outside.push_back({i, 0}); continue; }
+        /* a band wider than the matrix (ka > n - 1 is legal LAPACK storage) holds nothing beyond n - 1 */
+        const int B = std::max(std::min(std::max(q.ka, q.kb), q.n - 1), BSP_KMIN - 1);
+        auto it = gid.find({q.n, B});
+        if (it == gid.end()) {
+            it = gid.insert({{q.n, B}, (int)h->groups.size()}).first;
+            h->groups.emplace_back();
+            members.emplace_back();
+            Group &G = h->groups.back();
+            G.band = true;
+            G.k = B + 1; G.B = B; G.n = q.n; G.nkp = q.n + G.k; G.ka = 1;
+            G.FS = 2 * B + 2;
+            G.npad = BSP_NPAD(G.n, B);
+            G.nrows = BSP_NROWS(G.npad, B);
+            G.xrows = G.npad + B + 1;
+            G.ldw = ((G.n + 31) / 32) * 32;
+        }
+        members[it->second].push_back(i);
+        ++ndesc;
+        nband += (size_t)(q.ka + 1 + q.kb + 1) * q.n;
+    }
+    /* staging: the descriptors of every pencil, group by group, then the packed bands */
+    const size_t ddesc = doubles_for<BspBandSrc>(ndesc), total = ddesc + nband;
+    if (total > h->h_stage_cap) {
+        if (h->h_stage) cudaFreeHost(h->h_stage);
+        h->h_stage = nullptr; h->h_stage_cap = 0;
+        CU(cudaHostAlloc((void **)&h->h_stage, sizeof(double) * total, cudaHostAllocDefault));
+        h->h_stage_cap = total;
+    }
+    {
+        BspBandSrc *desc = (BspBandSrc *)h->h_stage;
+        size_t d = 0, off = ddesc;
+        for (auto &mem : members)
+            for (int i : mem) {
+                const bsp_band_pencil &q = pens[i];
+                const bool up = is_upper(q.uplo);
+                BspBandSrc &s = desc[d++];
+                s.ka = q.ka; s.kb = q.kb; s.upper = up;
+                s.a_off = (long long)off;
+                band_pack(h->h_stage + off, q.AB, q.ldab, q.ka, q.n, up);
+                off += (size_t)(q.ka + 1) * q.n;
+                s.b_off = (long long)off;
+                band_pack(h->h_stage + off, q.BB, q.ldbb, q.kb, q.n, up);
+                off += (size_t)(q.kb + 1) * q.n;
+            }
+    }
+    double *d_stage = nullptr;
+    if ((rc = dev_alloc(h, &d_stage, total))) return rc;
+    struct StageGuard {   /* gives the staging buffer back to the pool on every exit */
+        bspatom_handle h; double *p; size_t count;
+        ~StageGuard() { cudaStreamSynchronize(h->st); dev_free(h, p, count); }
+    } stage_guard{h, d_stage, total};
+    if (total) CU(cudaMemcpyAsync(d_stage, h->h_stage, sizeof(double) * total, cudaMemcpyHostToDevice, h->st));
+    std::vector<std::vector<int>> pd(h->groups.size());
+    size_t d = 0;
+    for (size_t gi = 0; gi < h->groups.size(); ++gi) {
+        Group &G = h->groups[gi];
+        G.ninst = (int)members[gi].size();
+        const size_t per_mat = (size_t)G.nrows * G.FS;
+        if ((rc = dev_alloc(h, &G.d_fbS, per_mat * G.ninst))) return rc;
+        if ((rc = dev_alloc(h, &G.d_fbH0, per_mat * G.ninst))) return rc;
+        if ((rc = dev_alloc(h, &G.d_fbQ, per_mat * G.ninst))) return rc;
+        if ((rc = dev_alloc(h, &G.d_pdinfo, G.ninst))) return rc;
+        const unsigned grid = (unsigned)((G.nrows + BSP_INGEST_TR - 1) / BSP_INGEST_TR) * (unsigned)G.ninst;
+        bsp_band_ingest_kernel<<<grid, BSP_INGEST_THREADS, 0, h->st>>>(d_stage, (const BspBandSrc *)d_stage + d, G.n, G.B,
+                                                                     G.nrows, G.d_fbS, G.d_fbH0, G.d_fbQ);
+        h->launches++;
+        CU(cudaGetLastError());
+        d += (size_t)G.ninst;
+        if ((rc = launch_pdcheck(h, G, h->st))) return rc;
+        pd[gi].resize(G.ninst);
+        CU(cudaMemcpyAsync(pd[gi].data(), G.d_pdinfo, sizeof(int) * G.ninst, cudaMemcpyDeviceToHost, h->st));
+    }
+    CU(cudaStreamSynchronize(h->st));
+    std::vector<Group> kept;
+    for (size_t gi = 0; gi < h->groups.size(); ++gi) {
+        Group &G = h->groups[gi];
+        for (int s = 0; s < G.ninst; ++s) {
+            const int i = members[gi][s];
+            if (pd[gi][s]) { h->outside.push_back({i, G.n + pd[gi][s]}); continue; }
+            G.prob_index.push_back(i);
+            G.inst.push_back(s);
+            G.nvec.push_back(pens[i].nvec);
+            G.cl.push_back(0.0);
+            G.coff.push_back(G.c_elems);
+            G.c_elems += (long long)G.n * pens[i].nvec;
+        }
+        G.npencil = (int)G.prob_index.size();
+        if (G.npencil == 0) { free_group(h, G); continue; }
+        kept.push_back(G);
+    }
+    h->groups = kept;
+    for (auto &G : h->groups)
+        if ((rc = upload_group_pencils(h, G))) return rc;
+    h->uploaded = true;
+    return 0;
+}
+
+int bspatom_solve_band_batch(bspatom_handle h, int nprob, const bsp_band_pencil *pens, double *E, double *C, int *info)
+{
+    const double t0 = host_ms();
+    int rc = bspatom_band_upload(h, nprob, pens);
+    if (rc) return rc;
+    return run_and_download(h, E, C, info, t0);
 }
 
 /* ------------------------------------------------------------------------- */

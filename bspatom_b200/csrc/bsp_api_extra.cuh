@@ -135,7 +135,19 @@ __global__ void bsp_verify_gram_kernel(int n, const int *__restrict__ nvec, cons
 }
 
 bspatom_handle g_level0 = nullptr;
-std::mutex g_level0_mu;   /* the LAPACK-shaped entry shares one lazily created handle: calls are serialised */
+std::mutex g_level0_mu;   /* the LAPACK-shaped entries share one lazily created handle: calls are serialised */
+
+/* that handle, created on the current device on first use (call with g_level0_mu held); nullptr and *info set on failure */
+bspatom_handle level0_handle(int *info)
+{
+    if (!g_level0) {
+        int dev = 0;
+        if (cudaGetDevice(&dev) != cudaSuccess) { *info = -100 - BSPATOM_ENODEVICE; return nullptr; }
+        int rc = bspatom_create(&g_level0, dev);
+        if (rc) { *info = -100 - rc; return nullptr; }
+    }
+    return g_level0;
+}
 
 } // namespace
 
@@ -350,6 +362,7 @@ int bspatom_wavefunction_resident(bspatom_handle h, int iprob, int ivec0, int nv
     int rc = check_device(h);
     if (rc) return rc;
     if (!h->ran) { h->err = "wavefunction_resident before a run"; return BSPATOM_ESTATE; }
+    if (h->band) { h->err = "wavefunction_resident: a band batch has no knots"; return BSPATOM_ESTATE; }
     Group *G = nullptr;
     int p = 0;
     if (iprob < 0 || iprob >= h->nprob || !find_resident(h, iprob, G, p)) return -2;
@@ -708,13 +721,8 @@ void bspatom_dsygv_(const int *itype, const char *jobz, const char *uplo, const 
     if (!w) { *info = -9; return; }
     if (n == 0) return;
     std::lock_guard<std::mutex> level0_lock(g_level0_mu);
-    if (!g_level0) {
-        int dev = 0;
-        if (cudaGetDevice(&dev) != cudaSuccess) { *info = -100 - BSPATOM_ENODEVICE; return; }
-        int rc = bspatom_create(&g_level0, dev);
-        if (rc) { *info = -100 - rc; return; }
-    }
-    bspatom_handle h = g_level0;
+    bspatom_handle h = level0_handle(info);
+    if (!h) return;
     auto a = [&](const double *M, int ld, int i, int j) -> double {   /* symmetric read of the stored triangle */
         if (upper) return (i <= j) ? M[(size_t)j * ld + i] : M[(size_t)i * ld + j];
         return (i >= j) ? M[(size_t)j * ld + i] : M[(size_t)i * ld + j];
@@ -830,6 +838,52 @@ void bspatom_dsygv_(const int *itype, const char *jobz, const char *uplo, const 
             else Bmat[(size_t)j * ldb + (j + i)] = v;
         }
     *info = bad;
+}
+
+/*
+ * DSBGV-shaped entry: one pencil through bspatom_solve_band_batch on the shared handle.  Arguments are checked in
+ * DSBGV's order (info = -i); AB and BB are only read.
+ */
+void bspatom_dsbgv_(const char *jobz, const char *uplo, const int *n_, const int *ka_, const int *kb_, double *AB,
+                    const int *ldab_, double *BB, const int *ldbb_, double *w, double *Z, const int *ldz_, double *work,
+                    int *info, ...)
+{
+    (void)work;
+    if (!info) return;
+    *info = 0;
+    const bool wantz = jobz && (*jobz == 'V' || *jobz == 'v');
+    const bool upper = uplo && is_upper(*uplo);
+    const int n = n_ ? *n_ : -1, ka = ka_ ? *ka_ : -1, kb = kb_ ? *kb_ : -1;
+    const int ldab = ldab_ ? *ldab_ : 0, ldbb = ldbb_ ? *ldbb_ : 0, ldz = ldz_ ? *ldz_ : 0;
+    if (!jobz || !(wantz || *jobz == 'N' || *jobz == 'n')) { *info = -1; return; }
+    if (!uplo || !(upper || *uplo == 'L' || *uplo == 'l')) { *info = -2; return; }
+    if (n < 0) { *info = -3; return; }
+    if (ka < 0 || ka > BSP_KMAX - 1) { *info = -4; return; }
+    if (kb < 0 || kb > ka) { *info = -5; return; }
+    if (!AB) { *info = -6; return; }
+    if (ldab < ka + 1) { *info = -7; return; }
+    if (!BB) { *info = -8; return; }
+    if (ldbb < kb + 1) { *info = -9; return; }
+    if (!w) { *info = -10; return; }
+    if (wantz && !Z) { *info = -11; return; }
+    if (ldz < 1 || (wantz && ldz < n)) { *info = -12; return; }
+    if (n == 0) return;
+    if (!band_finite(AB, ldab, ka, n, upper)) { *info = -6; return; }
+    if (!band_finite(BB, ldbb, kb, n, upper)) { *info = -8; return; }
+    std::lock_guard<std::mutex> level0_lock(g_level0_mu);
+    bspatom_handle h = level0_handle(info);
+    if (!h) return;
+    const bsp_band_pencil p = {n, ka, kb, upper ? 'U' : 'L', AB, ldab, BB, ldbb, wantz ? n : 0};
+    std::vector<double> E((size_t)n), Cv(wantz ? (size_t)n * n : 0);
+    int pinfo = 0;
+    const int rc = bspatom_solve_band_batch(h, 1, &p, E.data(), wantz ? Cv.data() : nullptr, &pinfo);
+    free_batch(h);
+    if (rc) { *info = -100 - rc; return; }
+    *info = pinfo;
+    if (pinfo > n) return;   /* B not positive definite: nothing was solved */
+    memcpy(w, E.data(), sizeof(double) * n);
+    if (wantz)
+        for (int j = 0; j < n; ++j) memcpy(Z + (size_t)j * ldz, Cv.data() + (size_t)j * n, sizeof(double) * n);
 }
 
 } /* extern "C" */

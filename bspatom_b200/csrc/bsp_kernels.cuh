@@ -650,6 +650,53 @@ __global__ void bsp_combine_kernel(double *fbH, const double *fbH0, const double
     fbH[(size_t)p * per_mat + i] = fma(cl[p], fbQ[src], fbH0[src]);
 }
 
+/* Where pencil p's bands sit in the staging buffer of bspatom_band_upload: A and B packed column-major with leading
+ * dimensions ka+1 and kb+1, in the caller's LAPACK layout (upper: AB(k+1+i-j, j), lower: AB(1+i-j, j), 1-based). */
+struct BspBandSrc {
+    long long a_off, b_off;   /* offsets in doubles */
+    int ka, kb, upper;
+};
+
+#define BSP_INGEST_TR 32        /* full-band rows per block */
+#define BSP_INGEST_THREADS 128
+
+/* A(i, j) of a symmetric band read from its stored triangle (0-based, |i - j| <= k) */
+__device__ __forceinline__ double bsp_band_at(const double *__restrict__ M, int k, int upper, int i, int j)
+{
+    const int lo = min(i, j), hi = max(i, j);
+    return upper ? M[(size_t)hi * (k + 1) + k + lo - hi] : M[(size_t)lo * (k + 1) + hi - lo];
+}
+
+/* caller-supplied bands -> full-band rows fb[i*FS + c] = M(i, i-B+c) of S (from B) and H0 (from A), Q = 0, padded
+ * exactly as bsp_assemble_kernel pads: rows n..nrows-1 hold diag(H0) = 1 and 0 elsewhere, column 2B+1 is 0.
+ * grid = ceil(nrows / BSP_INGEST_TR) * npencil blocks along x (row tiles of pencil 0, then of pencil 1, ...: a batch
+ * of many small pencils is not limited by the 65535 blocks of grid.y); pencil p becomes instance p of the group. */
+__global__ void __launch_bounds__(BSP_INGEST_THREADS) bsp_band_ingest_kernel(const double *__restrict__ stage,
+                                                                             const BspBandSrc *__restrict__ src, int n, int B,
+                                                                             int nrows, double *fbS, double *fbH0, double *fbQ)
+{
+    const int ntiles = (nrows + BSP_INGEST_TR - 1) / BSP_INGEST_TR;
+    const int p = blockIdx.x / ntiles, FS = 2 * B + 2;
+    const BspBandSrc s = src[p];
+    const int i0 = (blockIdx.x % ntiles) * BSP_INGEST_TR;
+    const int nout = min(BSP_INGEST_TR, nrows - i0) * FS;
+    const size_t base = ((size_t)p * nrows + i0) * FS;
+    for (int o = threadIdx.x; o < nout; o += BSP_INGEST_THREADS) {
+        const int i = i0 + o / FS, c = o % FS, j = i - B + c;
+        double a = 0.0, b = 0.0;
+        if (i < n && c <= 2 * B && j >= 0 && j < n) {
+            const int d = abs(i - j);
+            if (d <= s.ka) a = bsp_band_at(stage + s.a_off, s.ka, s.upper, i, j);
+            if (d <= s.kb) b = bsp_band_at(stage + s.b_off, s.kb, s.upper, i, j);
+        } else if (i >= n && c == B) {
+            a = 1.0;   /* padding row: decoupled, positive pivot */
+        }
+        fbS[base + o] = b;
+        fbH0[base + o] = a;
+        fbQ[base + o] = 0.0;
+    }
+}
+
 /* S positive definite?  one thread per instance walks the LDL^T pivots of S with the register-window
  * recurrence of the Sturm count (H := S, sigma = 0).  pd_info as below. */
 template <int B>

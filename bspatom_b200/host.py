@@ -22,7 +22,7 @@ from typing import Iterable, List, Optional, Sequence
 import numpy as np
 
 from . import _lib
-from ._lib import BspAtomError, BspProblem
+from ._lib import BspAtomError, BspBandPencil, BspProblem
 
 POT_COULOMB, POT_ROGERS, POT_SIMONS_FUES, POT_YUKAWA, POT_TIETZ, POT_TABLE = 0, 1, 2, 10, 11, -1
 
@@ -369,6 +369,39 @@ class BspAtom(BspInputs):
 
     def batch_run(self):
         _lib.check(self.lib, self._h, self.lib.bspatom_batch_run(self._h), "bspatom_batch_run")
+
+    # ---- caller-supplied band pencils (DSBGV semantics) ---------------------------------
+    def band_upload(self, pencils: Iterable, nvec=None, uplo: str = "U"):
+        """bspatom_band_upload: pencils are (AB, BB) or (AB, BB, uplo) with AB (ka+1, n) and BB (kb+1, n) in LAPACK
+        band storage (see band_pencil_array).  batch_run / batch_download / batch_verify / selection /
+        dipole_chain_resident then apply as after batch_upload."""
+        arr, keep, ns, _ = band_pencil_array(pencils, nvec, uplo)   # keep: the arrays arr points into
+        rc = self.lib.bspatom_band_upload(self._h, len(ns), arr)
+        _lib.check(self.lib, self._h, rc, "bspatom_band_upload")
+        self._last_items = ns
+
+    def solve_band_batch(self, pencils: Iterable, nvec=None, want_vectors: bool = True, uplo: str = "U",
+                         out_E: Optional[np.ndarray] = None, out_C: Optional[np.ndarray] = None):
+        """bspatom_solve_band_batch: A x = E B x for every (AB, BB[, uplo]) pencil.  Returns (list of E arrays, list of
+        (n, nvec) C blocks, info) like solve_batch; a pencil with info > n (B not positive definite) keeps whatever
+        its E / C slots held.  Pinned out_E / out_C (pinned_empty) are filled chunk by chunk."""
+        arr, keep, ns, nvs = band_pencil_array(pencils, nvec, uplo)   # keep: the arrays arr points into
+        nfs, nvs = np.asarray(ns, dtype=np.int64), np.asarray(nvs, dtype=np.int64)
+        self._last_items = ns
+        E = out_E if out_E is not None else pinned_empty(int(nfs.sum()))
+        Cbuf = (out_C if out_C is not None else pinned_empty(int((nfs * nvs).sum()))) if want_vectors else None
+        info = np.zeros(len(ns), dtype=np.int32)
+        rc = self.lib.bspatom_solve_band_batch(self._h, len(ns), arr, E.ctypes.data_as(C.c_void_p),
+                                               Cbuf.ctypes.data_as(C.c_void_p) if Cbuf is not None else None,
+                                               info.ctypes.data_as(C.c_void_p))
+        _lib.check(self.lib, self._h, rc, "bspatom_solve_band_batch")
+        eo = np.concatenate(([0], np.cumsum(nfs)))
+        co = np.concatenate(([0], np.cumsum(nfs * nvs)))
+        Es = [E[eo[i]:eo[i + 1]] for i in range(len(ns))]
+        Cs = []
+        if Cbuf is not None:
+            Cs = [Cbuf[co[i]:co[i + 1]].reshape((int(nfs[i]), int(nvs[i])), order="F") for i in range(len(ns))]
+        return Es, Cs, info
 
     def batch_download(self, E: np.ndarray, Cbuf: Optional[np.ndarray], info: np.ndarray):
         rc = self.lib.bspatom_batch_download(self._h, E.ctypes.data_as(C.c_void_p),
@@ -804,6 +837,84 @@ class _ProblemArray:
 
     def __getitem__(self, i):
         return self._as_parameter_[i]
+
+
+def _band_operand(M, what: str):
+    """(k+1, n) band in LAPACK storage -> (float64 array the pointer points into, leading dimension).  A Fortran-ordered
+    float64 view with a longer column stride (AB = buf[:ka+1, :] of a (ldab, n) buffer) is passed as it is, with that
+    stride as the leading dimension; anything else is copied into Fortran order."""
+    M = np.asarray(M)
+    if M.ndim != 2:
+        raise ValueError("%s must be a 2-D band array of shape (k+1, n), got %d dimensions" % (what, M.ndim))
+    if (M.dtype == np.float64 and M.strides[0] == 8 and M.shape[0] >= 1 and
+            (M.shape[1] <= 1 or (M.strides[1] % 8 == 0 and M.strides[1] >= 8 * M.shape[0]))):
+        return M, (M.strides[1] // 8 if M.shape[1] > 1 else M.shape[0])
+    M = np.asfortranarray(M, dtype=np.float64)
+    return M, max(1, M.shape[0])
+
+
+def band_pencil_array(pencils: Iterable, nvec=None, uplo: str = "U"):
+    """(AB, BB) / (AB, BB, uplo) list -> (struct bsp_band_pencil[], arrays it points into, n per pencil, nvec per
+    pencil).  Operands that are not Fortran-ordered float64 are copied; the struct array holds a reference to every
+    array it points into (a ctypes pointer stored in a struct does not keep its numpy array alive).  The half bandwidths are the band arrays' row counts minus one; the library checks their range, the
+    leading dimensions, uplo's value and nvec.  nvec: None (every eigenvector), an int (capped at each n) or one
+    value per pencil (passed as given)."""
+    pens = list(pencils)
+    if nvec is None or isinstance(nvec, (int, np.integer)):
+        per = [None if nvec is None else int(nvec)] * len(pens)
+        cap = True
+    else:
+        per = [int(v) for v in nvec]
+        cap = False
+        if len(per) != len(pens):
+            raise ValueError("nvec has %d entries for %d pencils" % (len(per), len(pens)))
+    arr = (BspBandPencil * max(1, len(pens)))()
+    keep, ns, nvs = [], [], []
+    for i, pen in enumerate(pens):
+        if len(pen) not in (2, 3):
+            raise ValueError("pencil %d: expected (AB, BB) or (AB, BB, uplo)" % i)
+        up = pen[2] if len(pen) == 3 else uplo
+        if not isinstance(up, str) or len(up) != 1:
+            raise ValueError("pencil %d: uplo must be one character, 'U' or 'L'" % i)
+        AB, ldab = _band_operand(pen[0], "AB")
+        BB, ldbb = _band_operand(pen[1], "BB")
+        if AB.shape[1] != BB.shape[1]:
+            raise ValueError("pencil %d: AB has %d columns, BB %d" % (i, AB.shape[1], BB.shape[1]))
+        n = AB.shape[1]
+        nv = n if per[i] is None else (min(per[i], n) if cap else per[i])
+        keep += [AB, BB]
+        p = arr[i]
+        p.n, p.ka, p.kb, p.uplo = n, AB.shape[0] - 1, BB.shape[0] - 1, up.encode()
+        p.AB, p.ldab = AB.ctypes.data_as(C.POINTER(C.c_double)), ldab
+        p.BB, p.ldbb = BB.ctypes.data_as(C.POINTER(C.c_double)), ldbb
+        p.nvec = nv
+        ns.append(n)
+        nvs.append(nv)
+    arr._keep = keep
+    return arr, keep, ns, nvs
+
+
+def dsbgv(AB: np.ndarray, BB: np.ndarray, jobz: str = "V", uplo: str = "U"):
+    """LAPACK-shaped entry ``bspatom_dsbgv_``: A x = w B x for one band pencil, AB (ka+1, n) and BB (kb+1, n) in LAPACK
+    band storage.  Returns (w, Z, info); Z is None for jobz = 'N'.  AB and BB are only read."""
+    lib = _lib.load()
+    A, ldab = _band_operand(AB, "AB")
+    Bm, ldbb = _band_operand(BB, "BB")
+    if A.shape[1] != Bm.shape[1]:
+        raise ValueError("AB has %d columns, BB %d" % (A.shape[1], Bm.shape[1]))
+    n = A.shape[1]
+    wantz = jobz in ("V", "v")
+    w = np.zeros(n)
+    Z = np.zeros((n, n), order="F") if wantz else None      # not referenced for jobz = 'N'
+    work = np.zeros(max(1, 3 * n))
+    ci = lambda v: C.byref(C.c_int(v))
+    info = C.c_int(0)
+    lib.bspatom_dsbgv_(jobz.encode(), uplo.encode(), ci(n), ci(A.shape[0] - 1), ci(Bm.shape[0] - 1),
+                       A.ctypes.data_as(C.c_void_p), ci(ldab), Bm.ctypes.data_as(C.c_void_p), ci(ldbb),
+                       w.ctypes.data_as(C.c_void_p), Z.ctypes.data_as(C.c_void_p) if wantz else None,
+                       ci(max(1, n) if wantz else 1),
+                       work.ctypes.data_as(C.c_void_p), C.byref(info))
+    return w, Z, info.value
 
 
 def dsygv(H: np.ndarray, S: np.ndarray, jobz: str = "V", uplo: str = "U"):

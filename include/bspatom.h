@@ -164,6 +164,49 @@ int bspatom_get_selection(bspatom_handle h, int *nsel);
  * otherwise verify after gathering Hij (matrices.f90:248) -- without moving the eigenvectors.           */
 int bspatom_batch_verify(bspatom_handle h, double *out4);
 
+/* ---- caller-supplied banded pencils (DSBGV semantics), batched ---------------- *
+ * A x = lambda B x for pencils the caller assembled (a model or core-polarisation term added to Hij, another banded
+ * discretisation such as FEM or Numerov), stored in LAPACK band storage.  The library keeps no pointer after a call. */
+typedef struct bsp_band_pencil {
+    int n;                 /* order, >= 0                                                  */
+    int ka, kb;            /* half bandwidths of A and B, 0..9 (BSP_KMAX - 1)               */
+    char uplo;             /* 'U': AB(ka+1+i-j, j) = A(i,j), max(1,j-ka) <= i <= j  (LAPACK)
+                              'L': AB(1+i-j, j)    = A(i,j), j <= i <= min(n,j+ka)          */
+    const double *AB; int ldab;   /* ldab >= ka+1, column-major (ldab, n)                    */
+    const double *BB; int ldbb;   /* ldbb >= kb+1                                            */
+    int nvec;              /* leading eigenvectors wanted, 0..n                             */
+} bsp_band_pencil;
+
+/* bspatom_band_upload takes the place of bspatom_batch_upload for a batch of band pencils; bspatom_batch_run,
+ * bspatom_batch_download, bspatom_batch_verify, bspatom_get_selection and bspatom_dipole_chain_resident then work
+ * unchanged.  bspatom_solve_band_batch is upload + run + download, with the E / C / info layout of
+ * bspatom_solve_batch (offsets by n and nvec in the caller's order; pinned E / C are filled chunk by chunk).
+ *  - Pencils are grouped by (n, B), B = max(min(max(ka, kb), n - 1), 2); narrower bands are zero-padded.  Each pencil is its own
+ *    instance with c_l = 0 and Q = 0, so the solver sees H = A exactly.  Only the stored triangle is read.
+ *  - Returns -3 for a malformed pencil (n < 0, ldab / ldbb too small, NULL AB / BB when n > 0, uplo not U / L,
+ *    nvec outside 0..n, or a NaN / Inf in a stored band) before any device work, BSPATOM_EUNSUPPORTED for ka or
+ *    kb > 9; bspatom_last_error names the pencil.
+ *  - info[p] as for bspatom_solve_batch: n + i when B is not positive definite at pivot i (dpotrf / dpbtrf
+ *    numbering), 1..n when that many eigenpairs missed the tolerance or form numerically degenerate pairs.
+ *    B is checked during the upload: a pencil that fails never reaches the solver and its E / C slots are not
+ *    written.  A pencil with n = 0 has info 0 and empty slots.
+ *  - No knots: bspatom_wavefunction_resident returns BSPATOM_ESTATE after a band upload, and sign_rule = 1 (the
+ *    literal CHKPHS) is skipped; every eigenvector gets the first-significant-coefficient-positive sign.
+ *  - No device-side state selection (sel_mode): nvec only.                                                       */
+int bspatom_band_upload(bspatom_handle h, int nprob, const bsp_band_pencil *pens);
+int bspatom_solve_band_batch(bspatom_handle h, int nprob, const bsp_band_pencil *pens, double *E, double *C,
+                             int *info);
+
+/* LAPACK DSBGV on the batched band path (one pencil).  Arguments are checked in DSBGV's order and an invalid one
+ * gives info = -i (also -4 for ka > 9, -6 / -8 for a NaN / Inf in the stored band of AB / BB).  On exit w is
+ * ascending and, with jobz = 'V', Z(:, j) is eigenvector j, Z^T B Z = I, signs as for bspatom_solve_batch.  Unlike
+ * LAPACK, AB and BB are left unchanged (no split-Cholesky factor is formed) and work is not used.  info > 0 as for
+ * bspatom_solve_band_batch; -100 - code for a device error.  Calls share one handle and are serialised with
+ * bspatom_dsygv_.  Trailing hidden CHARACTER lengths passed by Fortran compilers are ignored.                    */
+void bspatom_dsbgv_(const char *jobz, const char *uplo, const int *n, const int *ka, const int *kb,
+                    double *AB, const int *ldab, double *BB, const int *ldbb, double *w,
+                    double *Z, const int *ldz, double *work, int *info, ...);
+
 /* ---- LAPACK-compatible entry: one-token rename at matrices.f90:248 --------- *
  * DSYGV semantics for itype=1, jobz='V'|'N', uplo='U'|'L'.  The pencil must be
  * banded (bandwidth found from the zero pattern; the reference's matrices have
