@@ -393,7 +393,6 @@ struct GpuExec {
     double *cand_s;
     int *cand_c;
     int open_ok = 0;
-    int cur_iter = 0;
     bool ckpt = false;   /* iterations 0 and 1 run check-pointed (no stored factor) */
     cudaEvent_t ev_refine = nullptr; /* recorded between the bracketing and the refinement */
     cudaError_t first_err = cudaSuccess;
@@ -431,12 +430,20 @@ struct GpuExec {
         if (ev_refine) cudaEventRecord(ev_refine, h->st);
         bsp_prepare_kernel<<<grid(), BSP_EIG_THREADS, 0, h->st>>>(g); note();
     }
+    /* iteration 0 solves for the hashed start vector, 1 for S x, later ones for (H - rho S) x */
+    template <int RHS>
+    void factor_rhs(int it, int optional) {
+        if constexpr (RHS != BSP_RHS_RESID) {
+            if (ckpt && !optional) { bsp_factor_ckpt_kernel<B, RHS><<<grid(), BSP_EIG_THREADS, 0, h->st>>>(g); return; }
+        }
+        if (optional) bsp_factor_kernel<B, RHS><<<grid_listed(), LISTED_THREADS, 0, h->st>>>(g, it, optional);
+        else bsp_factor_kernel<B, RHS><<<grid(), BSP_EIG_THREADS, 0, h->st>>>(g, it, optional);
+    }
     void factor(int it, int optional) {
-        cur_iter = it;
         const int s = timed_begin(h, 1);
-        if (ckpt && it < 2 && !optional) bsp_factor_ckpt_kernel<B><<<grid(), BSP_EIG_THREADS, 0, h->st>>>(g, it);
-        else if (optional) bsp_factor_kernel<B><<<grid_listed(), LISTED_THREADS, 0, h->st>>>(g, it, optional);
-        else bsp_factor_kernel<B><<<grid(), BSP_EIG_THREADS, 0, h->st>>>(g, it, optional);
+        if (it == 0) factor_rhs<BSP_RHS_START>(it, optional);
+        else if (it == 1) factor_rhs<BSP_RHS_SX>(it, optional);
+        else factor_rhs<BSP_RHS_RESID>(it, optional);
         note();
         timed_end(h, s);
     }
@@ -453,12 +460,6 @@ struct GpuExec {
             bsp_back_kernel<B><<<grid(), BSP_EIG_THREADS, 0, h->st>>>(g, it, cn, cx, optional);
         }
         note();
-        timed_end(h, s);
-    }
-    void resid(int optional) {
-        const int s = timed_begin(h, 2);
-        /* runs in front of the factor pass of iteration cur_iter + 1 and follows the same list */
-        bsp_resid_kernel<B><<<grid_listed(), LISTED_THREADS, 0, h->st>>>(g, cur_iter + 1, optional); note();
         timed_end(h, s);
     }
     void check(int it, int select) { bsp_check_kernel<<<grid(), BSP_EIG_THREADS, 0, h->st>>>(g, it, select); note(); }
@@ -483,7 +484,7 @@ struct Carver {
 };
 
 struct ChunkPtrs {
-    double *fbH, *pbound, *lo, *hi, *samp_s, *gap, *sigma, *rho, *rho_prev, *scale, *res, *L, *X, *R, *cand_s, *fac;
+    double *fbH, *pbound, *lo, *hi, *samp_s, *gap, *sigma, *rho, *rho_prev, *scale, *res, *L, *X, *cand_s, *fac;
     double *samp_fm, *flm, *fhm, *beta, *xmax, *res2, *CK;
     int *clo, *chi, *samp_c, *done, *status, *counters, *cand_c, *samp_fe, *fle, *fhe, *side, *olist, *ocount, *rlist, *rcount;
 };
@@ -512,7 +513,6 @@ size_t carve_chunk(const Group &G, int np, char *base, ChunkPtrs &c, bool ckpt)
     c.L = cv.take<double>((size_t)np * G.npad * (G.B + 1) * G.ldw);
     c.CK = ckpt ? cv.take<double>((size_t)np * (G.npad / BSP_CK_STEPS(G.B)) * BSP_CK_DOUBLES(G.B) * G.ldw) : nullptr;
     c.X = cv.take<double>((size_t)np * G.xrows * G.ldw);
-    c.R = cv.take<double>((size_t)np * G.xrows * G.ldw);
     return cv.used;
 }
 
@@ -542,7 +542,7 @@ int enqueue_chunk_b(bspatom_handle h, Group &G, int p0, int np, const ChunkPtrs 
     g.samp_s = c.samp_s; g.samp_c = c.samp_c; g.gap = c.gap; g.done = c.done;
     g.samp_fm = c.samp_fm; g.samp_fe = c.samp_fe; g.flm = c.flm; g.fhm = c.fhm; g.fle = c.fle; g.fhe = c.fhe; g.side = c.side; g.beta = c.beta;
     g.sigma = c.sigma; g.rho = c.rho; g.rho_prev = c.rho_prev; g.scale = c.scale; g.res = c.res; g.xmax = c.xmax;
-    g.status = c.status; g.L = c.L; g.CK = c.CK; g.X = c.X; g.R = c.R; g.counters = c.counters;
+    g.status = c.status; g.L = c.L; g.CK = c.CK; g.X = c.X; g.counters = c.counters;
     g.olist = c.olist; g.ocount = c.ocount; g.res2 = c.res2; g.rlist = c.rlist; g.rcount = c.rcount;
     g.tau = h->opt.tau; g.delta_rel = h->opt.delta_rel; g.conv_tol = h->opt.conv_tol; g.vec_tol = h->opt.vec_tol;
 

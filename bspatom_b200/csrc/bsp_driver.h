@@ -16,7 +16,6 @@
  *   void factor(int iter, int optional);      // F pass (optional: compacted to the eigenpairs the last check listed,
  *                                             //         skipped once everything converged)
  *   void back(int iter, int corr_now, int corr_next, int optional);
- *   void resid(int optional);                 // residual of the listed vectors against their own Rayleigh quotient
  *   void check(int iter, int select);         // convergence marks, compaction list of what is left, bookkeeping
  */
 #ifndef BSP_DRIVER_H
@@ -50,15 +49,15 @@ inline void bsp_enqueue_chunk(Exec &ex, const BspSchedule &sch)
      * keeps in the iteration what misses conv_tol or has ||r||_2 / gap > vec_tol (bsp_check_converged): 10-17 % of
      * the eigenpairs of the N = 1000 pencils.  The passes from there on are COMPACTED to that list
      * (bsp_listed_index), so the correction pass that brings the S-orthogonality of neighbouring vectors from ~1e-8
-     * to ~1e-12 costs what its eigenpairs cost.  Compacted passes do not write the next right-hand side (scattered
-     * 8-byte stores): a residual pass over the list (band matvec only, no factor traffic) rebuilds
-     * r = (H - rho S) x with the current quotient in front of every correction. */
+     * to ~1e-12 costs what its eigenpairs cost.  No pass writes a right-hand side: every factor pass forms its own
+     * from the vector in X (S x, or r = (H - rho S) x) while it walks the band rows.  A back sweep followed by the
+     * check leaves the quotient and shift a correction after it needs: r against its new quotient, the shift delta
+     * away from that (bsp_back_finish). */
     const bool select = sch.min_iters <= 2;
     for (int t = 0; t < sch.max_iters; ++t) {
         const int optional = (t >= sch.min_iters);
         const bool check_follows = (t + 1 == sch.min_iters && select);
         const bool lean = select && optional;
-        if (lean) ex.resid(1);
         ex.factor(t, optional);
         ex.back(t, t >= 2, (check_follows || lean) ? -1 : (t + 1 >= 2), optional);
         /* check: 1 = residual / gap test that selects the correction pass; 2 = the looser one after a correction (not

@@ -3,7 +3,7 @@
  * bsp_core.h plus the small data-movement kernels (band combine, transpose).
  * Thread mapping everywhere: blockIdx.y = pencil, blockIdx.x*blockDim.x +
  * threadIdx.x = eigen index e, so a warp streams 32 consecutive e of one
- * pencil: every workspace access X/R/L[row][e] is a fully coalesced 256 B
+ * pencil: every workspace access X/L[row][e] is a fully coalesced 256 B
  * line.  The band rows of the pencil, which every thread of a block walks in the
  * same order, come through shared-memory tiles filled by bulk copies (BspRowsStaged).
  */
@@ -122,11 +122,11 @@ struct BspRowsStaged {
     using T = BspTile<B, G>;
     static constexpr bool GL = false;
     static constexpr int TR = T::TR;
-    static constexpr int RHS_RING = RING;   /* groups of the right-hand side in flight (factor kernel) */
+    static constexpr int RHS_RING = RING;   /* groups of right-hand-side look-ahead in flight (factor kernel) */
     double *sm;
     uint64_t *bars;   /* two mbarriers, count 1, not used by an earlier sweep of this launch */
     const double *gH, *gS;
-    double *rq = nullptr;   /* this thread's column of the right-hand-side ring: rq[slot_row * blockDim.x] */
+    double *rq = nullptr;   /* this thread's column of the look-ahead ring: rq[slot_row * blockDim.x] */
 #if defined(BSP_DEBUG)
     int dbg_issued = 0, dbg_acquired = 0;   /* thread 0: tiles issued / acquired so far (each stage: issue -> acquire -> release) */
 #endif
@@ -382,7 +382,7 @@ __global__ void bsp_prepare_kernel(BspEigChunk g)
 }
 
 #ifndef BSP_RHS_RING
-#define BSP_RHS_RING 3   /* groups of B+1 right-hand-side rows in flight per thread in the factor kernel */
+#define BSP_RHS_RING 3   /* groups of B+1 rows of x in flight per thread in the factor kernel */
 #endif
 /* wide bands: fewer groups, so that tiles + ring stay within the 48 KB of static shared memory */
 __host__ __device__ constexpr int bsp_rhs_ring(int B) { return B <= 6 ? BSP_RHS_RING : (B == 7 ? (BSP_RHS_RING < 2 ? BSP_RHS_RING : 2) : 1); }
@@ -405,7 +405,8 @@ __device__ __forceinline__ bool bsp_refine_map(const BspEigChunk &g, int p, int 
     return true;
 }
 
-template <int B>
+/* RHS: BSP_RHS_* (bsp_factor_forward_rhs) */
+template <int B, int RHS>
 __global__ void __launch_bounds__(BSP_EIG_THREADS, bsp_minb(BSP_MINB_FACTOR, B)) bsp_factor_kernel(BspEigChunk g, int iter, int optional)
 {
     __shared__ __align__(128) double sm[BspTile<B>::SMEM_DOUBLES];
@@ -422,7 +423,7 @@ __global__ void __launch_bounds__(BSP_EIG_THREADS, bsp_minb(BSP_MINB_FACTOR, B))
     constexpr int FS = 2 * B + 2;
     BspRowsStaged<B, RING> src{sm, bars, g.fbH + (size_t)p * g.nrows * FS, g.fbS + (size_t)g.inst[p] * g.nrows * FS};
     src.rq = ring + threadIdx.x;
-    bsp_factor_forward_rows<B>(g, p, e, ls, iter, active, src);
+    bsp_factor_forward_rhs<B, RHS>(g, p, e, ls, active, src);
 }
 
 template <int B>
@@ -443,8 +444,8 @@ __global__ void __launch_bounds__(BSP_EIG_THREADS, bsp_minb(BSP_MINB_BACK, B)) b
 }
 
 /* ---- check-pointed solves (full-width iterations 0 and 1) ---------------------------------------------------- */
-template <int B>
-__global__ void __launch_bounds__(BSP_EIG_THREADS, bsp_minb(BSP_MINB_FACTOR, B)) bsp_factor_ckpt_kernel(BspEigChunk g, int iter)
+template <int B, int RHS>
+__global__ void __launch_bounds__(BSP_EIG_THREADS, bsp_minb(BSP_MINB_FACTOR, B)) bsp_factor_ckpt_kernel(BspEigChunk g)
 {
     __shared__ __align__(128) double sm[BspTile<B>::SMEM_DOUBLES];
     constexpr int RING = bsp_rhs_ring(B);
@@ -457,7 +458,7 @@ __global__ void __launch_bounds__(BSP_EIG_THREADS, bsp_minb(BSP_MINB_FACTOR, B))
     constexpr int FS = 2 * B + 2;
     BspRowsStaged<B, RING> src{sm, bars, g.fbH + (size_t)p * g.nrows * FS, g.fbS + (size_t)g.inst[p] * g.nrows * FS};
     src.rq = ring + threadIdx.x;
-    bsp_factor_forward_rows<B, true>(g, p, e, e, iter, active, src);
+    bsp_factor_forward_rhs<B, RHS, true>(g, p, e, e, active, src);
 }
 
 /* scratch of the check-pointed back sweep: one column of shared memory per thread (slot i at base[i * blockDim.x]:
@@ -502,32 +503,13 @@ __global__ void __launch_bounds__(BSP_CKB_THREADS, BSP_CKB_MINB) bsp_back_ckpt_k
     bsp_back_ckpt_rows<B>(g, p, e, e, iter, corr_next, active, src, scr);
 }
 
-/* residual of the vectors in X against their own Rayleigh quotient, in front of a compacted correction pass: the
- * threads follow the list the last convergence check wrote (iteration `iter` reads the list of iter - 1) */
-template <int B>
-__global__ void __launch_bounds__(BSP_EIG_THREADS, bsp_minb(BSP_MINB_BACK, B)) bsp_resid_kernel(BspEigChunk g, int iter, int optional)
-{
-    __shared__ __align__(128) double sm[BspTile<B>::SMEM_DOUBLES];
-    __shared__ __align__(8) uint64_t bars[2];
-    if (optional && g.counters[BSP_C_REFINED]) return;
-    const int p = blockIdx.y, ls = blockIdx.x * blockDim.x + threadIdx.x;
-    int e;
-    bool active;
-    if (!bsp_refine_map(g, p, iter, optional && g.rlist != nullptr, e, active)) return;
-    bsp_stage_bars_init(bars);
-    if (!__syncthreads_or(active)) return;
-    constexpr int FS = 2 * B + 2;
-    BspRowsStaged<B> src{sm, bars, g.fbH + (size_t)p * g.nrows * FS, g.fbS + (size_t)g.inst[p] * g.nrows * FS};
-    bsp_back_substitute_rows<B, true>(g, p, e, ls, 0, 1, active, src);
-}
-
 __global__ void bsp_check_kernel(BspEigChunk g, int iter, int select)
 {
     if (g.counters[BSP_C_REFINED]) return;
     const int p = blockIdx.y, e = blockIdx.x * blockDim.x + threadIdx.x;
     const bool keep = bsp_check_keep(g, p, e, select);
     /* a warp appends its eigen indices as one ascending run (one atomic per warp): the compacted passes that
-     * follow then read X / R columns of neighbouring lanes from the same 32-byte sectors -- the selected pairs are
+     * follow then read X columns of neighbouring lanes from the same 32-byte sectors -- the selected pairs are
      * the ones with close neighbours and come in runs of consecutive indices */
     const unsigned mask = __ballot_sync(0xffffffffu, keep);
     if (mask) {
