@@ -23,6 +23,7 @@ EXPORTS = [
     "bspatom_create_multi", "bspatom_destroy_multi", "bspatom_last_error_multi", "bspatom_set_option_multi", "bspatom_solve_batch_multi",
     "bspatom_trans_amp_hermitian", "bspatom_assemble_zaij", "bspatom_wavefunction", "bspatom_wavefunction_resident", "bspatom_get_stats",
     "bspatom_band_upload", "bspatom_solve_band_batch", "bspatom_dsbgv_",
+    "bspatom_shifted_solve", "bspatom_shifted_solve_z", "bspatom_batch_sizes",
 ]
 
 
@@ -109,6 +110,9 @@ def load():
     L.bspatom_dsbgv_.argtypes = [C.c_char_p, C.c_char_p, _ip, _ip, _ip, C.c_void_p, _ip, C.c_void_p, _ip, C.c_void_p,
                                  C.c_void_p, _ip, C.c_void_p, _ip]
     L.bspatom_dsbgv_.restype = None
+    L.bspatom_batch_sizes.argtypes = [H, _ip, C.c_void_p]
+    for f in (L.bspatom_shifted_solve, L.bspatom_shifted_solve_z):
+        f.argtypes = [H, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     _lib = L
     return L
 

@@ -21,6 +21,7 @@
 #include <map>
 #include <string>
 #include <thread>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/bspatom.h"
@@ -50,6 +51,7 @@ struct Options {
     int trace = 0;        /* diagnostics: print the chunk / copy timeline of every run to stderr */
     int max_iters = 12;
     int chunk = 0; /* 0 = auto */
+    long long shifted_chunk = 0; /* systems per chunk of a shifted solve (0: as many as the workspace budget allows) */
     int workers = 2; /* concurrent chunk streams (1..4) */
     int stream_chunks = 6; /* chunks per group when results stream to the host */
     int stream_workers = 2; /* chunk streams when results stream to the host */
@@ -63,6 +65,8 @@ struct Group {
     int ninst = 0, npencil = 0;
     bool any_vtab = false;
     bool band = false; /* ingested from caller-supplied bands (bspatom_band_upload): no knots, nothing to assemble */
+    bool rows_built = false; /* S, H0, Q rows hold the assembly (a band group's from the upload); a shifted solve
+                                before the first batch_run assembles once, batch_run assembles every time as before */
     int budget_pencils = 0; /* pencils whose workspaces fit the memory budget (decided on the first run) */
     std::vector<int> prob_index; /* pencil -> caller's problem index */
     std::vector<int> inst, nvec;
@@ -125,7 +129,7 @@ struct bspatom_handle_s {
     long long c_bytes_copied = 0; /* eigenvector bytes the last run sent to the host */
     size_t budget_bytes = 0;      /* workspace budget of this handle (decided on the first run) */
     bool mail_info = false;       /* the mailbox holds pdinfo / bad of the last run (see run_internal) */
-    double stats[24] = {0};
+    double stats[27] = {0};
     long long launches = 0;
     /* further chunk streams: auxiliary contexts (own stream, workspace, event pool) that the same host
      * thread enqueues on, so several chunks are in flight and the GPU back-fills the tail waves and the
@@ -800,6 +804,7 @@ int bspatom_set_option(bspatom_handle h, const char *name, double v)
     else if (s == "first_check_round" || s == "check_every") { /* accepted and ignored: the schedule is static */ }
     else if (s == "chunk") h->opt.chunk = (int)v;
     else if (s == "vec_tol") h->opt.vec_tol = v;
+    else if (s == "shifted_chunk") h->opt.shifted_chunk = (long long)std::max(0.0, v);
     else if (s == "sign_rule") h->opt.sign_rule = (int)v;
     else if (s == "gemm_variant") bsp_gemm_force = (int)v;   /* process-wide: A/B runs of the contraction kernel only */
     else if (s == "ckpt") { h->opt.ckpt = (int)v; h->budget_bytes = 0; }
@@ -814,7 +819,7 @@ int bspatom_get_stats(bspatom_handle h, double *out, int nout)
 {
     if (!h) return -1;
     if (!out) return -2;
-    for (int i = 0; i < nout && i < 24; ++i) out[i] = h->stats[i];
+    for (int i = 0; i < nout && i < 27; ++i) out[i] = h->stats[i];
     return 0;
 }
 
@@ -1051,6 +1056,19 @@ int launch_pdcheck(bspatom_handle h, Group &G, cudaStream_t st)
     }
 }
 
+/* S, H0 and Q rows of every instance of an assembled group */
+int assemble_group(bspatom_handle h, Group &G)
+{
+    BspAsmArgs a;
+    memset(&a, 0, sizeof a);
+    a.n = G.n; a.nkp = G.nkp; a.ka = G.ka; a.nrows = G.nrows; a.ninst = G.ninst; a.want_pi = 0;
+    a.rt = G.d_rt; a.xgwg = G.d_xgwg; a.par = G.d_par; a.vtab = G.d_vtab;
+    a.fb[BSP_MAT_S] = G.d_fbS; a.fb[BSP_MAT_H0] = G.d_fbH0; a.fb[BSP_MAT_Q] = G.d_fbQ;
+    const int rc = launch_assembly(h, G.k, a);
+    if (!rc) G.rows_built = true;
+    return rc;
+}
+
 BspRunStats stats_from_report(const int *r)
 {
     BspRunStats st = {r[BSP_C_ROUNDS], r[BSP_C_ITERS], r[BSP_C_OPEN_END], r[BSP_C_CROWDED_END], r[BSP_C_UNCONV_END]};
@@ -1131,13 +1149,8 @@ int run_internal(bspatom_handle h, double *E_out, double *C_out)
         /* ---- assembly, once per instance ---- */
         CU(cudaEventRecord(e1, h->st));
         if (!G.band) {   /* a band group's rows were written by bspatom_band_upload */
-            BspAsmArgs a;
-            memset(&a, 0, sizeof a);
-            a.n = G.n; a.nkp = G.nkp; a.ka = G.ka; a.nrows = G.nrows; a.ninst = G.ninst; a.want_pi = 0;
-            a.rt = G.d_rt; a.xgwg = G.d_xgwg; a.par = G.d_par; a.vtab = G.d_vtab;
-            a.fb[BSP_MAT_S] = G.d_fbS; a.fb[BSP_MAT_H0] = G.d_fbH0; a.fb[BSP_MAT_Q] = G.d_fbQ;
             const int s = timed_begin(h, 3);
-            rc = launch_assembly(h, G.k, a);
+            rc = assemble_group(h, G);
             timed_end(h, s);
             if (rc) return rc;
         }
@@ -1480,6 +1493,17 @@ int bspatom_batch_download(bspatom_handle h, double *E, double *C, int *info)
     return 0;
 }
 
+int bspatom_batch_sizes(bspatom_handle h, int *nprob, int *n)
+{
+    int rc = check_device(h);
+    if (rc) return rc;
+    if (!nprob) return -2;
+    if (!h->uploaded) { h->err = "batch_sizes before batch_upload / band_upload"; return BSPATOM_ESTATE; }
+    *nprob = h->nprob;
+    if (n) std::copy(h->p_n.begin(), h->p_n.end(), n);
+    return 0;
+}
+
 int bspatom_get_selection(bspatom_handle h, int *nsel)
 {
     int rc = check_device(h);
@@ -1759,6 +1783,307 @@ int bspatom_assemble_band(bspatom_handle h, const bsp_problem *p, double *S, dou
             }
     }
     return 0;
+}
+
+} /* extern "C" */
+
+/* ---- driven equation (H - z S) x = b on the resident batch (bspatom_shifted_solve[_z]) ------------------------ */
+namespace {
+
+bool device_accessible(const void *p)
+{
+    cudaPointerAttributes at;
+    if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { cudaGetLastError(); return false; }
+    return at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged;
+}
+
+/* one chunk of a group's systems, laid out in slots (see BspShiftChunk) */
+struct ShiftChunkPlan {
+    std::vector<int> pen;              /* pencils of the group whose H_l the chunk forms, in row-block order */
+    std::vector<int> blk_pen;          /* per block: index into pen                                        */
+    std::vector<int> sys;              /* per slot: caller's system or -1                                  */
+};
+
+template <int B, class T>
+int enqueue_shifted_b(bspatom_handle h, const BspShiftChunk<T> &c, const long long *d_off, T *d_B, T *d_X, int *d_info_out,
+                      double *d_berr_out)
+{
+    const int nblk = c.nslot / BSP_EIG_THREADS;
+    const dim3 lay((c.n + 31) / 32, (c.nslot + 31) / 32, (unsigned)c.nrhs), lay_t(32, 8);
+    if (c.nrhs > 0) { bsp_shifted_layout_kernel<T, true><<<lay, lay_t, 0, h->st>>>(c, d_off, d_B, c.Bv ? (T *)c.Bv : nullptr, nullptr); h->launches++; }
+    bsp_shifted_factor_kernel<B, T><<<nblk, BSP_EIG_THREADS, 0, h->st>>>(c);
+    h->launches++;
+    if (c.nrhs > 0) {
+        /* every step is enqueued up front: finished columns return at once (BspShiftChunk::done) */
+        const dim3 grid(nblk, 1, c.nrhs);
+        for (int step = 0; step <= BSP_SHIFT_MAXSTEPS + 1; ++step) {
+            bsp_shifted_forward_kernel<B, T><<<grid, BSP_EIG_THREADS, 0, h->st>>>(c, step);
+            if (step <= BSP_SHIFT_MAXSTEPS) bsp_shifted_back_kernel<B, T><<<grid, BSP_EIG_THREADS, 0, h->st>>>(c, step);
+            h->launches += 2;
+        }
+    }
+    bsp_shifted_report_kernel<T><<<nblk, BSP_EIG_THREADS, 0, h->st>>>(c, d_info_out, d_berr_out);
+    h->launches++;
+    if (c.nrhs > 0) { bsp_shifted_layout_kernel<T, false><<<lay, lay_t, 0, h->st>>>(c, d_off, d_X, c.X, d_info_out); h->launches++; }
+    CU(cudaGetLastError());
+    return 0;
+}
+
+template <class T>
+int enqueue_shifted(bspatom_handle h, int B, const BspShiftChunk<T> &c, const long long *d_off, T *d_B, T *d_X, int *d_info_out,
+                    double *d_berr_out)
+{
+    switch (B) {
+    case 2: return enqueue_shifted_b<2, T>(h, c, d_off, d_B, d_X, d_info_out, d_berr_out);
+    case 3: return enqueue_shifted_b<3, T>(h, c, d_off, d_B, d_X, d_info_out, d_berr_out);
+    case 4: return enqueue_shifted_b<4, T>(h, c, d_off, d_B, d_X, d_info_out, d_berr_out);
+    case 5: return enqueue_shifted_b<5, T>(h, c, d_off, d_B, d_X, d_info_out, d_berr_out);
+    case 6: return enqueue_shifted_b<6, T>(h, c, d_off, d_B, d_X, d_info_out, d_berr_out);
+    case 7: return enqueue_shifted_b<7, T>(h, c, d_off, d_B, d_X, d_info_out, d_berr_out);
+    case 8: return enqueue_shifted_b<8, T>(h, c, d_off, d_B, d_X, d_info_out, d_berr_out);
+    case 9: return enqueue_shifted_b<9, T>(h, c, d_off, d_B, d_X, d_info_out, d_berr_out);
+    default: return BSPATOM_EUNSUPPORTED;
+    }
+}
+
+/* device bytes of a chunk: per slot (factor, x, Y, b, state) and per pencil (its H_l rows) */
+template <class T>
+size_t shift_slot_bytes(const Group &G, int nrhs)
+{
+    return sizeof(T) * ((size_t)G.n * (G.B + 1) + 3 * (size_t)G.n * nrhs) + (size_t)nrhs * (4 + 8 + 8) + 2 * 8 + 8 + 4 * 3 + 8;
+}
+
+template <class T>
+int shifted_solve(bspatom_handle h, int nsys, const int *iprob, const double *z, int nrhs, const T *Bm, T *Xm, int *info,
+                  double *berr)
+{
+    constexpr bool CPLX = std::is_same<T, BspZ>::value;
+    int rc = check_device(h);
+    if (rc) return rc;
+    /* every check before any device work: a rejected call leaves the handle as it was */
+    if (nsys < 0) return -2;
+    if (nsys > 0 && !iprob) return -3;
+    if (nsys > 0 && !z) return -4;
+    if (nrhs < 0 || nrhs > 65535) return -5;
+    const bool any_rhs = (long long)nsys * nrhs > 0;
+    if (any_rhs && !Bm) return -6;
+    if (any_rhs && !Xm) return -7;
+    if (nsys > 0 && !info) return -8;
+    if (!h->uploaded) { h->err = "shifted_solve before batch_upload / band_upload"; return BSPATOM_ESTATE; }
+    for (int s = 0; s < nsys; ++s) {
+        if (iprob[s] < 0 || iprob[s] >= h->nprob) { h->err = "iprob[" + std::to_string(s) + "] out of range"; return -3; }
+        const double zr = z[CPLX ? 2 * s : s], zi = CPLX ? z[2 * s + 1] : 0.0;
+        if (!std::isfinite(zr) || !std::isfinite(zi)) { h->err = "z of system " + std::to_string(s) + " is not finite"; return -4; }
+    }
+    /* where each caller problem lives: (group, pencil), or outside every group with its upload info */
+    std::vector<int> pg(h->nprob, -1), pp(h->nprob, -1), pinfo(h->nprob, 0);
+    for (auto &o : h->outside) pinfo[o.first] = o.second;
+    for (size_t gi = 0; gi < h->groups.size(); ++gi)
+        for (int p = 0; p < h->groups[gi].npencil; ++p) { pg[h->groups[gi].prob_index[p]] = (int)gi; pp[h->groups[gi].prob_index[p]] = p; }
+    std::vector<long long> off(nsys + 1, 0);
+    for (int s = 0; s < nsys; ++s) off[s + 1] = off[s] + (long long)h->p_n[iprob[s]] * nrhs;
+    for (int s = 0; s < nsys; ++s)
+        if (pg[iprob[s]] < 0) { info[s] = pinfo[iprob[s]]; if (berr) berr[s] = 0.0; }
+    const size_t total = (size_t)off[nsys];
+    h->stats[24] = 0.0; h->stats[25] = 0.0; h->stats[26] = 0.0;
+
+    struct Bufs {   /* gives every device buffer of the call back to the pool on every exit */
+        bspatom_handle h;
+        std::vector<std::pair<void *, size_t>> v;
+        ~Bufs() { cudaStreamSynchronize(h->st); for (auto &b : v) h->pool.insert({pool_round(b.second), b.first}), h->pool_bytes += pool_round(b.second); }
+    } bufs{h};
+    auto take = [&](auto **p, size_t count) -> int {
+        using E = typename std::remove_reference<decltype(**p)>::type;
+        const int r = dev_alloc(h, p, count);
+        if (!r) bufs.v.push_back({(void *)*p, (count ? count : 1) * sizeof(E)});
+        return r;
+    };
+    T *d_B = nullptr, *d_X = nullptr;
+    const bool b_dev = total > 0 && device_accessible(Bm), x_dev = total > 0 && device_accessible(Xm);
+    if (total > 0) {
+        if (b_dev) d_B = const_cast<T *>(Bm);
+        else {
+            if ((rc = take(&d_B, total))) return rc;
+            CU(cudaMemcpyAsync(d_B, Bm, total * sizeof(T), cudaMemcpyDefault, h->st));
+        }
+        if (x_dev) d_X = Xm;
+        else if ((rc = take(&d_X, total))) return rc;
+    }
+    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+    CU(cudaEventCreate(&ev0));
+    struct EvGuard { cudaEvent_t &a, &b; ~EvGuard() { if (a) cudaEventDestroy(a); if (b) cudaEventDestroy(b); } } evg{ev0, ev1};
+    CU(cudaEventCreate(&ev1));
+    float ms_total = 0.0f;
+    int steps_max = 0;
+    unsigned long long corrections = 0;
+    std::vector<char> solved(nsys, 0);   /* X_s was written */
+
+    size_t budget = h->budget_bytes;
+    if (budget == 0) {
+        size_t free_b = 0, total_b = 0;
+        CU(cudaMemGetInfo(&free_b, &total_b));
+        budget = std::max<size_t>(std::min<size_t>((free_b + h->ws.bytes + h->pool_bytes) / 2, (size_t)64 << 30), 1);
+    }
+    constexpr int NT = BSP_EIG_THREADS;
+    for (size_t gi = 0; gi < h->groups.size(); ++gi) {
+        Group &G = h->groups[gi];
+        std::vector<int> mine;
+        for (int s = 0; s < nsys; ++s) if (pg[iprob[s]] == (int)gi) mine.push_back(s);
+        if (mine.empty()) continue;
+        std::stable_sort(mine.begin(), mine.end(), [&](int a, int b) { return pp[iprob[a]] < pp[iprob[b]]; });
+        if (!G.band && !G.rows_built && (rc = assemble_group(h, G))) return rc;
+        /* blocks of NT slots, each on one pencil; chunks of whole blocks within the workspace budget */
+        const size_t per_mat = (size_t)G.nrows * G.FS;
+        const size_t slot_b = shift_slot_bytes<T>(G, nrhs), pen_b = per_mat * sizeof(double) + 64;
+        /* the layout kernels' grid.y counts tiles of 32 slots: at most 65535 of them per chunk */
+        const long long max_slots = (65535LL * 32 / NT) * NT;
+        const long long cap_sys = std::min<long long>(h->opt.shifted_chunk > 0 ? h->opt.shifted_chunk : max_slots, max_slots);
+        std::vector<ShiftChunkPlan> plans(1);
+        size_t bytes = 0;
+        for (size_t i = 0; i < mine.size();) {
+            const int p = pp[iprob[mine[i]]];
+            size_t j = i;
+            while (j < mine.size() && pp[iprob[mine[j]]] == p && (long long)(j - i) < NT) ++j;   /* one block */
+            ShiftChunkPlan *pl = &plans.back();
+            const bool new_pen = pl->pen.empty() || pl->pen.back() != p;
+            const size_t add = NT * slot_b + (new_pen ? pen_b : 0);
+            const long long used_sys = (long long)pl->blk_pen.size() * NT;
+            if (!pl->blk_pen.empty() && (bytes + add > budget || used_sys + NT > cap_sys)) {
+                plans.emplace_back();
+                pl = &plans.back();
+                bytes = 0;
+            }
+            if (pl->pen.empty() || pl->pen.back() != p) { pl->pen.push_back(p); bytes += pen_b; }
+            pl->blk_pen.push_back((int)pl->pen.size() - 1);
+            for (size_t k = i; k < j; ++k) pl->sys.push_back(mine[k]);
+            for (size_t k = j - i; k < (size_t)NT; ++k) pl->sys.push_back(-1);
+            bytes += NT * slot_b;
+            i = j;
+        }
+        for (auto &pl : plans) {
+            const int nslot = (int)pl.sys.size(), npen = (int)pl.pen.size(), nblk = nslot / NT;
+            /* per-chunk tables, one host-to-device copy */
+            std::vector<double> zr(nslot, 0.0), zi(nslot, 0.0), cl(npen);
+            std::vector<long long> soff(nslot, 0);
+            std::vector<int> ints;   /* blk_inst[nblk], sys[nslot], pen_inst[npen] */
+            for (int b = 0; b < nblk; ++b) ints.push_back(G.inst[pl.pen[pl.blk_pen[b]]]);
+            for (int k = 0; k < nslot; ++k) {
+                const int s = pl.sys[k];
+                ints.push_back(s);
+                if (s < 0) continue;
+                zr[k] = z[CPLX ? 2 * s : s];
+                zi[k] = CPLX ? z[2 * s + 1] : 0.0;
+                soff[k] = off[s];
+            }
+            for (int q = 0; q < npen; ++q) { ints.push_back(G.inst[pl.pen[q]]); cl[q] = G.cl[pl.pen[q]]; }
+            ints.insert(ints.end(), pl.blk_pen.begin(), pl.blk_pen.end());
+            Carver cv{nullptr};
+            auto carve = [&](char *base, BspShiftChunk<T> &c, double *&d_z, double *&d_cl, long long *&d_off, int *&d_ints,
+                             int *&d_info_out, double *&d_berr_out, double *&d_fbH) {
+                cv = Carver{base};
+                d_fbH = cv.take<double>((size_t)npen * per_mat);
+                c.L = cv.take<T>((size_t)G.n * (G.B + 1) * nslot);
+                c.X = cv.take<T>((size_t)G.n * nrhs * nslot);
+                c.Y = cv.take<T>((size_t)G.n * nrhs * nslot);
+                c.Bv = cv.take<T>((size_t)G.n * nrhs * nslot);
+                d_z = cv.take<double>(2 * (size_t)nslot);
+                d_cl = cv.take<double>(npen);
+                d_off = cv.take<long long>(nslot);
+                d_ints = cv.take<int>(ints.size());
+                c.info = cv.take<int>(nslot);
+                c.done = cv.take<int>((size_t)nrhs * nslot);
+                c.berr = cv.take<double>((size_t)nrhs * nslot);
+                c.bprev = cv.take<double>((size_t)nrhs * nslot);
+                c.steps = cv.take<int>(1);
+                c.corrections = cv.take<unsigned long long>(1);
+                d_info_out = cv.take<int>(nslot);
+                d_berr_out = cv.take<double>(nslot);
+                return cv.used;
+            };
+            BspShiftChunk<T> c;
+            memset(&c, 0, sizeof c);
+            double *d_z, *d_cl, *d_berr_out, *d_fbH;
+            long long *d_off;
+            int *d_ints, *d_info_out;
+            const size_t need = carve(nullptr, c, d_z, d_cl, d_off, d_ints, d_info_out, d_berr_out, d_fbH);
+            if ((rc = ensure_workspace(h, need))) return rc;
+            carve(h->ws.base, c, d_z, d_cl, d_off, d_ints, d_info_out, d_berr_out, d_fbH);
+            std::vector<double> zz(zr);
+            zz.insert(zz.end(), zi.begin(), zi.end());
+            CU(cudaMemcpyAsync(d_z, zz.data(), sizeof(double) * zz.size(), cudaMemcpyHostToDevice, h->st));
+            CU(cudaMemcpyAsync(d_cl, cl.data(), sizeof(double) * npen, cudaMemcpyHostToDevice, h->st));
+            CU(cudaMemcpyAsync(d_off, soff.data(), sizeof(long long) * nslot, cudaMemcpyHostToDevice, h->st));
+            CU(cudaMemcpyAsync(d_ints, ints.data(), sizeof(int) * ints.size(), cudaMemcpyHostToDevice, h->st));
+            CU(cudaMemsetAsync(c.steps, 0, sizeof(int), h->st));
+            CU(cudaMemsetAsync(c.corrections, 0, sizeof(unsigned long long), h->st));
+            const int *d_blk_inst = d_ints, *d_sys = d_ints + nblk, *d_pen_inst = d_sys + nslot, *d_blk_pen = d_pen_inst + npen;
+            c.n = G.n; c.npad = G.npad; c.nslot = nslot; c.nrhs = nrhs; c.nrows = G.nrows;
+            c.fbH = d_fbH; c.fbS = G.d_fbS; c.blk_pen = d_blk_pen; c.blk_inst = d_blk_inst; c.sys = d_sys;
+            c.zr = d_z; c.zi = d_z + nslot;
+            CU(cudaEventRecord(ev0, h->st));
+            {
+                /* H_l of the chunk's pencils, as bsp_combine_kernel forms it for the eigen stages */
+                dim3 grid((unsigned)((per_mat + 255) / 256), npen);
+                bsp_combine_kernel<<<grid, 256, 0, h->st>>>(d_fbH, G.d_fbH0, G.d_fbQ, d_pen_inst, d_cl, per_mat);
+                h->launches++;
+            }
+            if ((rc = enqueue_shifted<T>(h, G.B, c, d_off, d_B, d_X, d_info_out, d_berr_out))) return rc;
+            CU(cudaEventRecord(ev1, h->st));
+            std::vector<int> iout(nslot);
+            std::vector<double> bout(nslot);
+            int st = 0;
+            unsigned long long corr = 0;
+            CU(cudaMemcpyAsync(iout.data(), d_info_out, sizeof(int) * nslot, cudaMemcpyDeviceToHost, h->st));
+            CU(cudaMemcpyAsync(bout.data(), d_berr_out, sizeof(double) * nslot, cudaMemcpyDeviceToHost, h->st));
+            CU(cudaMemcpyAsync(&st, c.steps, sizeof(int), cudaMemcpyDeviceToHost, h->st));
+            CU(cudaMemcpyAsync(&corr, c.corrections, sizeof corr, cudaMemcpyDeviceToHost, h->st));
+            CU(cudaStreamSynchronize(h->st));
+            float ms = 0.0f;
+            CU(cudaEventElapsedTime(&ms, ev0, ev1));
+            ms_total += ms;
+            steps_max = std::max(steps_max, st);
+            corrections += corr;
+            for (int k = 0; k < nslot; ++k) {
+                const int s = pl.sys[k];
+                if (s < 0) continue;
+                info[s] = iout[k];
+                if (berr) berr[s] = bout[k];
+                solved[s] = (iout[k] == 0 || iout[k] == G.n + 1);
+            }
+        }
+    }
+    if (total > 0 && !x_dev) {
+        /* the solutions that were written, in runs of consecutive systems */
+        int s = 0;
+        while (s < nsys) {
+            if (!solved[s] || off[s + 1] == off[s]) { ++s; continue; }
+            int q = s;
+            while (q + 1 < nsys && solved[q + 1]) ++q;
+            CU(cudaMemcpyAsync(Xm + off[s], d_X + off[s], sizeof(T) * (size_t)(off[q + 1] - off[s]), cudaMemcpyDefault, h->st));
+            s = q + 1;
+        }
+        CU(cudaStreamSynchronize(h->st));
+    }
+    h->stats[24] = ms_total;
+    h->stats[25] = steps_max;
+    h->stats[26] = (double)corrections;
+    return 0;
+}
+
+} // namespace
+
+extern "C" {
+
+int bspatom_shifted_solve(bspatom_handle h, int nsys, const int *iprob, const double *z, int nrhs, const double *B, double *X,
+                          int *info, double *berr)
+{
+    return shifted_solve<double>(h, nsys, iprob, z, nrhs, B, X, info, berr);
+}
+
+int bspatom_shifted_solve_z(bspatom_handle h, int nsys, const int *iprob, const double *z, int nrhs, const double *B, double *X,
+                            int *info, double *berr)
+{
+    return shifted_solve<BspZ>(h, nsys, iprob, z, nrhs, (const BspZ *)B, (BspZ *)X, info, berr);
 }
 
 } /* extern "C" */

@@ -629,7 +629,94 @@ __global__ void bsp_combine_kernel(double *fbH, const double *fbH0, const double
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= per_mat) return;
     const size_t src = (size_t)inst[p] * per_mat + i;
-    fbH[(size_t)p * per_mat + i] = fma(cl[p], fbQ[src], fbH0[src]);
+    fbH[(size_t)p * per_mat + i] = bsp_combine_entry(cl[p], fbQ[src], fbH0[src]);
+}
+
+/* ---- driven equation (H - z S) x = b (bsp_shifted_*_rows): one thread per system slot, blockIdx.z = right-hand
+ * side; a block's slots all belong to pencil blk_pen[blockIdx.x], whose band rows the block stages once ---------- */
+template <int B, class T>
+__global__ void __launch_bounds__(BSP_EIG_THREADS) bsp_shifted_factor_kernel(BspShiftChunk<T> c)
+{
+    __shared__ __align__(128) double sm[BspTile<B>::SMEM_DOUBLES];
+    __shared__ __align__(8) uint64_t bars[2];
+    const int slot = blockIdx.x * blockDim.x + threadIdx.x;
+    const bool active = slot < c.nslot && c.sys[slot] >= 0;
+    bsp_stage_bars_init(bars);
+    if (!__syncthreads_or(active)) return;
+    constexpr int FS = 2 * B + 2;
+    BspRowsStaged<B> src{sm, bars, c.fbH + (size_t)c.blk_pen[blockIdx.x] * c.nrows * FS,
+                         c.fbS + (size_t)c.blk_inst[blockIdx.x] * c.nrows * FS};
+    bsp_shifted_factor_rows<B, T>(c, slot, active, src);
+}
+
+template <int B, class T>
+__global__ void __launch_bounds__(BSP_EIG_THREADS) bsp_shifted_forward_kernel(BspShiftChunk<T> c, int step)
+{
+    __shared__ __align__(128) double sm[BspTile<B>::SMEM_DOUBLES];
+    __shared__ __align__(8) uint64_t bars[2];
+    const int slot = blockIdx.x * blockDim.x + threadIdx.x, col = blockIdx.z;
+    const bool active = bsp_shift_active(c, slot, col);   /* finished systems return */
+    bsp_stage_bars_init(bars);
+    if (!__syncthreads_or(active)) return;
+    constexpr int FS = 2 * B + 2;
+    BspRowsStaged<B> src{sm, bars, c.fbH + (size_t)c.blk_pen[blockIdx.x] * c.nrows * FS,
+                         c.fbS + (size_t)c.blk_inst[blockIdx.x] * c.nrows * FS};
+    bsp_shifted_forward_rows<B, T>(c, slot, col, step, active, src);
+}
+
+template <int B, class T>
+__global__ void __launch_bounds__(BSP_EIG_THREADS) bsp_shifted_back_kernel(BspShiftChunk<T> c, int step)
+{
+    const int slot = blockIdx.x * blockDim.x + threadIdx.x, col = blockIdx.z;
+    if (bsp_shift_active(c, slot, col)) bsp_shifted_back_rows<B, T>(c, slot, col, step);
+}
+
+template <class T>
+__global__ void bsp_shifted_report_kernel(BspShiftChunk<T> c, int *info_out, double *berr_out)
+{
+    bsp_shifted_report(c, blockIdx.x * blockDim.x + threadIdx.x, info_out, berr_out);
+}
+
+/* caller layout (system s: n x nrhs column-major at off[slot]) <-> slot-fastest workspace [col][row][slot], through
+ * 32 x 32 shared-memory tiles tile[slot][row]: the caller side is read or written along rows, the workspace side
+ * along slots, so both sides move whole lines.  The scatter writes only the systems whose solution is defined
+ * (info 0 or n + 1). */
+template <class T, bool GATHER>
+__global__ void bsp_shifted_layout_kernel(BspShiftChunk<T> c, const long long *off, T *caller, T *ws, const int *info)
+{
+    __shared__ T tile[32][33];
+    const int r0 = blockIdx.x * 32, s0 = blockIdx.y * 32, col = blockIdx.z, n = c.n;
+    const size_t ld = c.nslot;
+    /* caller side: lane = row, one system per step */
+    auto caller_ok = [&](int slot) {
+        if (slot >= c.nslot || c.sys[slot] < 0) return false;
+        if (GATHER) return true;
+        const int i = info[slot];
+        return i == 0 || i == n + 1;
+    };
+    if (GATHER) {
+        for (int ss = threadIdx.y; ss < 32; ss += blockDim.y) {
+            const int slot = s0 + ss, row = r0 + threadIdx.x;
+            if (row < n && caller_ok(slot)) tile[ss][threadIdx.x] = caller[off[slot] + (long long)col * n + row];
+        }
+    } else {   /* workspace side: lane = slot, one row per step */
+        for (int rr = threadIdx.y; rr < 32; rr += blockDim.y) {
+            const int row = r0 + rr, slot = s0 + threadIdx.x;
+            if (row < n && slot < c.nslot) tile[threadIdx.x][rr] = ws[((size_t)col * n + row) * ld + slot];
+        }
+    }
+    __syncthreads();
+    if (GATHER) {
+        for (int rr = threadIdx.y; rr < 32; rr += blockDim.y) {
+            const int row = r0 + rr, slot = s0 + threadIdx.x;
+            if (row < n && slot < c.nslot && c.sys[slot] >= 0) ws[((size_t)col * n + row) * ld + slot] = tile[threadIdx.x][rr];
+        }
+    } else {
+        for (int ss = threadIdx.y; ss < 32; ss += blockDim.y) {
+            const int slot = s0 + ss, row = r0 + threadIdx.x;
+            if (row < n && caller_ok(slot)) caller[off[slot] + (long long)col * n + row] = tile[ss][threadIdx.x];
+        }
+    }
 }
 
 /* Where pencil p's bands sit in the staging buffer of bspatom_band_upload: A and B packed column-major with leading

@@ -258,13 +258,13 @@ class BspAtom(BspInputs):
                    "bspatom_set_option")
 
     def stats(self) -> dict:
-        out = (C.c_double * 24)()
-        self.lib.bspatom_get_stats(self._h, out, 24)
+        out = (C.c_double * 27)()
+        self.lib.bspatom_get_stats(self._h, out, 27)
         keys = ["launches", "rounds", "iters", "ms_assembly", "ms_eigenvalues", "ms_eigenvectors", "ms_finalize",
                 "ms_total", "ms_k_round", "ms_k_factor", "ms_k_back", "ms_k_assembly",
                 "n_k_round", "n_k_factor", "n_k_back", "n_k_assembly", "wall_ms_upload", "wall_ms_run",
                 "wall_ms_download", "chunks_redone", "selected_third_solve", "wall_ms_copy_tail", "c_bytes_copied",
-                "ms_resident_contraction"]
+                "ms_resident_contraction", "ms_shifted_solve", "shifted_refinement_steps", "shifted_corrections"]
         return dict(zip(keys, list(out)))
 
     # ---- MATRIX_SVT (matrices.f90:1-200) ------------------------------------------------
@@ -602,6 +602,76 @@ def _wavefunction_resident(self, iprob: int, ivec0: int, nvec: int, ra: float, r
 
 BspAtom.dipole_chain_resident = _dipole_chain_resident
 BspAtom.wavefunction_resident = _wavefunction_resident
+
+
+def _shifted_solve(self, iprob, z, B):
+    """bspatom_shifted_solve[_z]: (A_p - z_s B_p) X_s = B_s for every system s on pencil p = iprob[s] of the uploaded
+    batch (batch_upload: A = H_l, B = S; band_upload: the caller's pencils).  B: one array per system, (n_p,) or
+    (n_p, nrhs) with the same nrhs for all.  A complex z or B selects the complex-symmetric solver.  Returns
+    (X, info, berr): X a list shaped like B (a system with info in 1..n or from the upload keeps NaN), info and berr
+    as in include/bspatom.h."""
+    iprob = np.ascontiguousarray(np.asarray(iprob, dtype=np.int32).reshape(-1))
+    nsys = len(iprob)
+    z = np.asarray(z).reshape(-1)
+    B = list(B)
+    if len(z) != nsys or len(B) != nsys:
+        raise ValueError("iprob, z and B must have one entry per system")
+    sizes = self.batch_sizes()
+    if np.any(iprob < 0) or np.any(iprob >= len(sizes)):
+        raise ValueError("iprob out of range")
+    cplx = np.iscomplexobj(z) or any(np.iscomplexobj(b) for b in B)
+    dt = np.complex128 if cplx else np.float64
+    vec = [np.ndim(b) == 1 for b in B]
+    mats = [np.asarray(b, dtype=dt).reshape(np.shape(b)[0], -1) for b in B]
+    nrhs = mats[0].shape[1] if nsys else 0
+    for s, M in enumerate(mats):
+        if M.shape != (sizes[iprob[s]], nrhs):
+            raise ValueError("B[%d] has shape %s, pencil %d needs (%d, %d)" % (s, M.shape, iprob[s], sizes[iprob[s]], nrhs))
+    flat = np.concatenate([M.ravel(order="F") for M in mats]) if nsys else np.zeros(0, dt)
+    flat = np.ascontiguousarray(flat)
+    X = np.full_like(flat, np.nan)
+    zz = np.ascontiguousarray(z.astype(dt))
+    info = np.zeros(nsys, dtype=np.int32)
+    berr = np.zeros(nsys)
+    f = self.lib.bspatom_shifted_solve_z if cplx else self.lib.bspatom_shifted_solve
+    rc = f(self._h, nsys, iprob.ctypes.data_as(C.c_void_p), zz.ctypes.data_as(C.c_void_p), nrhs,
+           flat.ctypes.data_as(C.c_void_p), X.ctypes.data_as(C.c_void_p), info.ctypes.data_as(C.c_void_p),
+           berr.ctypes.data_as(C.c_void_p))
+    _lib.check(self.lib, self._h, rc, "bspatom_shifted_solve")
+    out, o = [], 0
+    for s, M in enumerate(mats):
+        blk = X[o:o + M.size].reshape(M.shape, order="F")
+        out.append(blk[:, 0] if vec[s] else blk)
+        o += M.size
+    return out, info, berr
+
+
+def _shifted_solve_ptrs(self, iprob, z, nrhs: int, B_ptr: int, X_ptr: int, complex_: bool = False):
+    """bspatom_shifted_solve[_z] on raw (host or DEVICE) addresses of B and X, e.g. torch CUDA tensors' data_ptr()."""
+    iprob = np.ascontiguousarray(np.asarray(iprob, dtype=np.int32).reshape(-1))
+    zz = np.ascontiguousarray(np.asarray(z, dtype=np.complex128 if complex_ else np.float64).reshape(-1))
+    info = np.zeros(len(iprob), dtype=np.int32)
+    berr = np.zeros(len(iprob))
+    f = self.lib.bspatom_shifted_solve_z if complex_ else self.lib.bspatom_shifted_solve
+    rc = f(self._h, len(iprob), iprob.ctypes.data_as(C.c_void_p), zz.ctypes.data_as(C.c_void_p), int(nrhs),
+           C.c_void_p(B_ptr), C.c_void_p(X_ptr), info.ctypes.data_as(C.c_void_p), berr.ctypes.data_as(C.c_void_p))
+    _lib.check(self.lib, self._h, rc, "bspatom_shifted_solve")
+    return info, berr
+
+
+def _batch_sizes(self) -> np.ndarray:
+    """orders n of the problems of the resident batch, whichever call uploaded it (bspatom_batch_sizes)"""
+    nprob = C.c_int(0)
+    _lib.check(self.lib, self._h, self.lib.bspatom_batch_sizes(self._h, C.byref(nprob), None), "bspatom_batch_sizes")
+    n = np.zeros(nprob.value, dtype=np.int32)
+    _lib.check(self.lib, self._h, self.lib.bspatom_batch_sizes(self._h, C.byref(nprob), n.ctypes.data_as(C.c_void_p)),
+               "bspatom_batch_sizes")
+    return n
+
+
+BspAtom.batch_sizes = _batch_sizes
+BspAtom.shifted_solve = _shifted_solve
+BspAtom.shifted_solve_ptrs = _shifted_solve_ptrs
 
 
 class BspAtomMulti:

@@ -154,6 +154,10 @@ int bspatom_batch_download(bspatom_handle h, double *E, double *C, int *info);  
                                    (unified addressing: a device destination keeps the eigenpairs on the GPU, e.g. as the
                                    send buffer of the NCCL gather to the rank that runs the writers) */
 
+/* the resident batch of the last batch_upload / band_upload (or solve_batch / solve_band_batch): *nprob problems and,
+ * when n is not NULL, their orders n[nprob]; BSPATOM_ESTATE without one */
+int bspatom_batch_sizes(bspatom_handle h, int *nprob, int *n);
+
 /* eigenvectors computed per problem by the last run (= nvec unless sel_mode = 1): nsel[nprob] */
 int bspatom_get_selection(bspatom_handle h, int *nsel);
 
@@ -206,6 +210,36 @@ int bspatom_solve_band_batch(bspatom_handle h, int nprob, const bsp_band_pencil 
 void bspatom_dsbgv_(const char *jobz, const char *uplo, const int *n, const int *ka, const int *kb,
                     double *AB, const int *ldab, double *BB, const int *ldbb, double *w,
                     double *Z, const int *ldz, double *work, int *info, ...);
+
+/* ---- driven equation (A_p - z B_p) x = b on the resident batch, many shifts and pencils per call ------------- *
+ * Dalgarno-Lewis / Sternheimer equations, dynamic polarisabilities, resolvents on an energy grid, DGBSV-shaped solves
+ * of uploaded band pencils.  System s solves (A_p - z_s B_p) X_s = B_s on pencil p = iprob[s] (0-based) of the batch
+ * of the last bspatom_batch_upload (A_p = H_l, formed exactly as the eigen stages form it: fma(c_l, Q, H0); B_p = S)
+ * or bspatom_band_upload (the caller's A and B).  bspatom_batch_run is not needed first: an assembled batch is
+ * assembled once by the first shifted solve; the resident eigenpairs, selection and info are left as they were.
+ *  - bspatom_shifted_solve: real z[s], B, X.  bspatom_shifted_solve_z: complex z (z[2s], z[2s+1]), B and X
+ *    (COMPLEX*16, re / im interleaved); the matrix is complex symmetric (no conjugation).
+ *  - B, X: n_p x nrhs column-major blocks, back to back in system order, host or device pointers (unified
+ *    addressing).  Systems may name a pencil any number of times, in any order, and mix pencils of different shapes.
+ *  - Method: un-pivoted banded LDL^T of A - z B, then refinement in correction form as DGBRFS stops it: while the
+ *    componentwise backward error berr = max_i |r_i| / (|A - zB| |x| + |b|)_i (|.| = |re| + |im| for complex values,
+ *    as ZGBRFS) is above eps and halved in the last step, at most 5 corrections x += (A - zB)^-1 r, r = b - (A - zB) x.
+ *  - info[s]: 0 solved; i in 1..n: the pivot of row i is exactly zero or not finite (X_s not written); n + 1: the
+ *    refinement stopped with berr above 64 eps or not a number (a NaN or Inf in B_s; X_s written, berr[s] says how
+ *    far); for a pencil the band upload
+ *    dropped (B not positive definite) its upload info n + i, X_s untouched; a pencil with n = 0 has info 0.
+ *  - berr[s] (berr may be NULL): the largest backward error above over the columns of system s.
+ *  - Returns -i for a bad argument i (nsys < 0; iprob NULL or out of range; z NULL or not finite; nrhs outside
+ *    0..65535; B / X NULL with nsys * nrhs > 0; info NULL with nsys > 0) and BSPATOM_ESTATE without an uploaded
+ *    batch, all before any device work; the handle stays usable.  Option "shifted_chunk" caps the systems per chunk
+ *    (0, the default: as many as the workspace budget holds); results do not depend on the chunking.
+ *  - bspatom_get_stats: out[24] = device ms, out[25] = most corrections any column needed, out[26] = corrections
+ *    summed over all columns (last shifted solve).
+ *  - B and X must hold sum over s of n_p * nrhs values: bspatom_batch_sizes gives every n_p of the resident batch. */
+int bspatom_shifted_solve(bspatom_handle h, int nsys, const int *iprob, const double *z, int nrhs, const double *B,
+                          double *X, int *info, double *berr);
+int bspatom_shifted_solve_z(bspatom_handle h, int nsys, const int *iprob, const double *z, int nrhs, const double *B,
+                            double *X, int *info, double *berr);
 
 /* ---- LAPACK-compatible entry: one-token rename at matrices.f90:248 --------- *
  * DSYGV semantics for itype=1, jobz='V'|'N', uplo='U'|'L'.  The pencil must be
@@ -271,7 +305,11 @@ int bspatom_wavefunction_resident(bspatom_handle h, int iprob, int ivec0, int nv
  * iterations, out[3] ms in assembly, out[4] ms eigenvalue stage, out[5] ms
  * eigenvector stage, out[6] ms finalize, out[7] total device ms,
  * out[8..11] summed device ms of the multisection / factor / back-substitution /
- * assembly kernels (CUDA events around each launch), out[12..15] their launch counts */
+ * assembly kernels (CUDA events around each launch), out[12..15] their launch counts, out[16..18] host wall ms of
+ * upload / run / download, out[19] chunks redone, out[20] eigenpairs given a third solve, out[21] wall ms waiting for
+ * the last copies, out[22] eigenvector bytes copied, out[23] device ms of bspatom_dipole_chain_resident,
+ * out[24] device ms, out[25] most refinement corrections of one column and out[26] corrections summed over all
+ * columns, of the last bspatom_shifted_solve[_z] */
 int bspatom_get_stats(bspatom_handle h, double *out, int nout);
 
 #ifdef __cplusplus
