@@ -10,7 +10,7 @@ CSRC = os.path.join(_HERE, "csrc")
 LIB = os.path.join(_HERE, "libbspatom.so")
 LIB_DEBUG = os.path.join(_HERE, "libbspatom_debug.so")   # -DBSP_DEBUG: device-side bounds / pipeline asserts (tests only)
 SOURCES = ["bsp_api.cu"]
-HEADERS = ["bsp_api_extra.cuh", "bsp_assembly.cuh", "bsp_core.h", "bsp_driver.h", "bsp_gemm.cuh",
+HEADERS = ["bsp_api_extra.cuh", "bsp_assembly.cuh", "bsp_core.h", "bsp_driver.h", "bsp_gemm.cuh", "bsp_plan.h",
            "bsp_kernels.cuh", os.path.join("..", "..", "include", "bspatom.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared"]

@@ -30,11 +30,25 @@
 #include "bsp_driver.h"
 #include "bsp_gemm.cuh"
 #include "bsp_kernels.cuh"
+#include "bsp_plan.h"
 
 #define BSP_KMIN 3
 #define BSP_KMAX 10
 
+static_assert(BSP_PLAN_THREADS == BSP_EIG_THREADS, "the chunk plan sizes a wave in eigen-stage blocks");
+
 namespace {
+
+/* f(std::integral_constant<int, v>{}) for the one v in LO..HI that equals x: the kernels templated on that axis are
+ * instantiated for exactly these values; BSPATOM_EUNSUPPORTED for any other x */
+template <int LO, int HI, class F>
+int dispatch(int x, F &&f)
+{
+    if constexpr (LO > HI) return BSPATOM_EUNSUPPORTED;
+    else return x == LO ? f(std::integral_constant<int, LO>{}) : dispatch<LO + 1, HI>(x, f);
+}
+template <class F> int with_half_band(int B, F &&f) { return dispatch<BSP_KMIN - 1, BSP_KMAX - 1>(B, f); }
+template <class F> int with_order(int k, F &&f) { return dispatch<BSP_KMIN, BSP_KMAX>(k, f); }
 
 struct Options {
     double tau = 1e-4;
@@ -222,6 +236,27 @@ void free_group(bspatom_handle h, Group &g)
     g = Group();
 }
 
+/* row layout of a group's pencils: order n, half bandwidth B */
+void set_geometry(Group &G, int n, int B)
+{
+    G.n = n; G.B = B; G.FS = 2 * B + 2;
+    G.npad = BSP_NPAD(n, B);
+    G.nrows = BSP_NROWS(G.npad, B);
+    G.xrows = G.npad + B + 1;
+    G.ldw = ((n + 31) / 32) * 32;
+}
+
+/* S, H0 and Q rows of every instance of a group and their positive-definiteness info */
+int alloc_group_rows(bspatom_handle h, Group &G)
+{
+    const size_t per_mat = (size_t)G.nrows * G.FS;
+    int rc;
+    if ((rc = dev_alloc(h, &G.d_fbS, per_mat * G.ninst))) return rc;
+    if ((rc = dev_alloc(h, &G.d_fbH0, per_mat * G.ninst))) return rc;
+    if ((rc = dev_alloc(h, &G.d_fbQ, per_mat * G.ninst))) return rc;
+    return dev_alloc(h, &G.d_pdinfo, G.ninst);
+}
+
 void free_batch(bspatom_handle h)
 {
     for (auto &g : h->groups) free_group(h, g);
@@ -280,10 +315,6 @@ int validate_problem(const bsp_problem &p)
     if (p.sel_mode == 1 && (p.sel_extra < 0 || !(p.sel_ecut_a == p.sel_ecut_a) || !(p.sel_ecut_b == p.sel_ecut_b))) return -3;
     return 0;
 }
-
-struct InstKey {
-    const bsp_problem *p;
-};
 
 bool same_instance(const bsp_problem &a, const bsp_problem &b)
 {
@@ -355,38 +386,24 @@ void timed_collect(bspatom_handle h)
 }
 
 /* ---- assembly launch ---------------------------------------------------- */
-template <int K>
-int launch_assembly_k(bspatom_handle h, const BspAsmArgs &a)
-{
-    constexpr int PK = K * (K + 1) / 2;
-    const int per_int = (a.want_pi ? 6 : 4) * PK + (a.want_pi ? K * K : 0);
-    const size_t smem = (size_t)(BSP_ASM_TR + K - 1) * per_int * sizeof(double);
-    dim3 grid((a.nrows + BSP_ASM_TR - 1) / BSP_ASM_TR, a.ninst);
-    if (a.ka <= 16) {
-        CU(cudaFuncSetAttribute(bsp_assemble_kernel<K, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        bsp_assemble_kernel<K, 16><<<grid, BSP_ASM_THREADS, smem, h->st>>>(a);
-    } else {
-        CU(cudaFuncSetAttribute(bsp_assemble_kernel<K, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        bsp_assemble_kernel<K, 32><<<grid, BSP_ASM_THREADS, smem, h->st>>>(a);
-    }
-    h->launches++;
-    CU(cudaGetLastError());
-    return 0;
-}
-
 int launch_assembly(bspatom_handle h, int k, const BspAsmArgs &a)
 {
-    switch (k) {
-    case 3: return launch_assembly_k<3>(h, a);
-    case 4: return launch_assembly_k<4>(h, a);
-    case 5: return launch_assembly_k<5>(h, a);
-    case 6: return launch_assembly_k<6>(h, a);
-    case 7: return launch_assembly_k<7>(h, a);
-    case 8: return launch_assembly_k<8>(h, a);
-    case 9: return launch_assembly_k<9>(h, a);
-    case 10: return launch_assembly_k<10>(h, a);
-    default: return BSPATOM_EUNSUPPORTED;
-    }
+    return with_order(k, [&](auto K) {
+        constexpr int PK = K * (K + 1) / 2;
+        const int per_int = (a.want_pi ? 6 : 4) * PK + (a.want_pi ? K * K : 0);
+        const size_t smem = (size_t)(BSP_ASM_TR + K - 1) * per_int * sizeof(double);
+        dim3 grid((a.nrows + BSP_ASM_TR - 1) / BSP_ASM_TR, a.ninst);
+        if (a.ka <= 16) {
+            CU(cudaFuncSetAttribute(bsp_assemble_kernel<K, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            bsp_assemble_kernel<K, 16><<<grid, BSP_ASM_THREADS, smem, h->st>>>(a);
+        } else {
+            CU(cudaFuncSetAttribute(bsp_assemble_kernel<K, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            bsp_assemble_kernel<K, 32><<<grid, BSP_ASM_THREADS, smem, h->st>>>(a);
+        }
+        h->launches++;
+        CU(cudaGetLastError());
+        return 0;
+    });
 }
 
 /* ---- eigen stage executor ------------------------------------------------ */
@@ -469,10 +486,15 @@ struct GpuExec {
     void check(int it, int select) { bsp_check_kernel<<<grid(), BSP_EIG_THREADS, 0, h->st>>>(g, it, select); note(); }
 };
 
-struct ChunkTimes {
-    cudaEvent_t ev[4];
-    cudaEvent_t selected = nullptr;   /* owned by the caller; null when the group has no selection */
+/* one chunk of a run: pencils [p0, p0 + np) of a group, enqueued on chunk stream w; its events are the caller's */
+struct ChunkRec {
+    int p0 = 0, np = 0, w = 0;
+    cudaEvent_t ev[4];                /* start, refinement, finalize, end */
+    cudaEvent_t selected = nullptr;   /* null when the group has no selection */
     int *sel_report = nullptr;        /* device view of the selection mailbox slots of this chunk's pencils */
+    /* results streaming to the host: `done` is recorded on the chunk's stream behind its last kernel (timed only with
+     * the `trace` option, which also times the copy from c0 to c1) and the copy of its results waits for it */
+    cudaEvent_t done = nullptr, c0 = nullptr, c1 = nullptr;
 };
 
 /* carve the chunk workspace out of one allocation */
@@ -526,7 +548,7 @@ bool use_ckpt(bspatom_handle h, const Group &G) { return h->opt.ckpt > 0 || (h->
  * report: BSP_C_WORDS ints on the device that receive the chunk's control block at the end. */
 template <int B>
 int enqueue_chunk_b(bspatom_handle h, Group &G, int p0, int np, const ChunkPtrs &c, const BspSchedule &sch,
-                    ChunkTimes &tm, int *report)
+                    ChunkRec &tm, int *report)
 {
     const size_t per_mat = (size_t)G.nrows * G.FS;
     CU(cudaEventRecord(tm.ev[0], h->st));
@@ -581,12 +603,7 @@ int enqueue_chunk_b(bspatom_handle h, Group &G, int p0, int np, const ChunkPtrs 
         int maxnv = 0;
         for (int p = 0; p < np; ++p) maxnv = std::max(maxnv, G.nvec[p0 + p]);
         if (maxnv > 0 && h->opt.sign_rule == 1 && G.d_rt) {
-            switch (G.k) {
-#define BSP_CHK_CASE(K_) case K_: bsp_chkphs_kernel<K_><<<grid, BSP_EIG_THREADS, 0, h->st>>>(g, G.d_rt, G.nkp, c.fac); break;
-                BSP_CHK_CASE(3) BSP_CHK_CASE(4) BSP_CHK_CASE(5) BSP_CHK_CASE(6) BSP_CHK_CASE(7) BSP_CHK_CASE(8) BSP_CHK_CASE(9) BSP_CHK_CASE(10)
-#undef BSP_CHK_CASE
-            default: break;
-            }
+            with_order(G.k, [&](auto K) { bsp_chkphs_kernel<K><<<grid, BSP_EIG_THREADS, 0, h->st>>>(g, G.d_rt, G.nkp, c.fac); return 0; });
             h->launches++;
             CU(cudaGetLastError());
         }
@@ -605,19 +622,9 @@ int enqueue_chunk_b(bspatom_handle h, Group &G, int p0, int np, const ChunkPtrs 
 }
 
 int enqueue_chunk(bspatom_handle h, Group &G, int p0, int np, const ChunkPtrs &c, const BspSchedule &sch,
-                  ChunkTimes &tm, int *report)
+                  ChunkRec &tm, int *report)
 {
-    switch (G.B) {
-    case 2: return enqueue_chunk_b<2>(h, G, p0, np, c, sch, tm, report);
-    case 3: return enqueue_chunk_b<3>(h, G, p0, np, c, sch, tm, report);
-    case 4: return enqueue_chunk_b<4>(h, G, p0, np, c, sch, tm, report);
-    case 5: return enqueue_chunk_b<5>(h, G, p0, np, c, sch, tm, report);
-    case 6: return enqueue_chunk_b<6>(h, G, p0, np, c, sch, tm, report);
-    case 7: return enqueue_chunk_b<7>(h, G, p0, np, c, sch, tm, report);
-    case 8: return enqueue_chunk_b<8>(h, G, p0, np, c, sch, tm, report);
-    case 9: return enqueue_chunk_b<9>(h, G, p0, np, c, sch, tm, report);
-    default: return BSPATOM_EUNSUPPORTED;
-    }
+    return with_half_band(G.B, [&](auto B) { return enqueue_chunk_b<B>(h, G, p0, np, c, sch, tm, report); });
 }
 
 int ensure_workspace(bspatom_handle h, size_t bytes, bspatom_handle pool_owner = nullptr)
@@ -861,12 +868,8 @@ int bspatom_batch_upload(bspatom_handle h, int nprob, const bsp_problem *probs)
             ginsts.emplace_back();
             ghash.emplace_back();
             Group &G = h->groups.back();
-            G.k = p.k; G.B = p.k - 1; G.n = p.nfun; G.nkp = p.nkp; G.ka = p.ka;
-            G.FS = 2 * G.B + 2;
-            G.npad = BSP_NPAD(G.n, G.B);
-            G.nrows = BSP_NROWS(G.npad, G.B);
-            G.xrows = G.npad + G.B + 1;
-            G.ldw = ((G.n + 31) / 32) * 32;
+            G.k = p.k; G.nkp = p.nkp; G.ka = p.ka;
+            set_geometry(G, p.nfun, p.k - 1);
         } else {
             gi = it->second;
         }
@@ -919,11 +922,7 @@ int bspatom_batch_upload(bspatom_handle h, int nprob, const bsp_problem *probs)
         G.ninst = (int)ginsts[gi].size();
         G.npencil = (int)G.prob_index.size();
         if ((rc = upload_group_instances(h, G, ginsts[gi]))) return rc;
-        const size_t per_mat = (size_t)G.nrows * G.FS;
-        if ((rc = dev_alloc(h, &G.d_fbS, per_mat * G.ninst))) return rc;
-        if ((rc = dev_alloc(h, &G.d_fbH0, per_mat * G.ninst))) return rc;
-        if ((rc = dev_alloc(h, &G.d_fbQ, per_mat * G.ninst))) return rc;
-        if ((rc = dev_alloc(h, &G.d_pdinfo, G.ninst))) return rc;
+        if ((rc = alloc_group_rows(h, G))) return rc;
         if ((rc = upload_group_pencils(h, G))) return rc;
     }
     {
@@ -982,24 +981,28 @@ CopyQueue *copy_queue(int dev)
     return g_q[dev];
 }
 
-/* enqueue on `cs` the D2H of pencils [p0, p0+np) of group G into the caller's E / C */
-int copy_chunk_out(bspatom_handle h, Group &G, int p0, int np, double *E, double *C, cudaStream_t cs, const int *nsel = nullptr)
+/* enqueue on `cs` the D2H of pencils [p0, p0+np) of group G into the caller's E / C; c_bytes receives the bytes of
+ * eigenvectors enqueued */
+int copy_chunk_out(bspatom_handle h, Group &G, int p0, int np, double *E, double *C, cudaStream_t cs, const int *nsel,
+                   long long &c_bytes)
 {
+    c_bytes = 0;
     if (nsel) {
         /* device-side selection: E in merged runs, C problem by problem, the selected columns only (a prefix of the
          * problem's column-major block) */
-        int rc = copy_chunk_out(h, G, p0, np, E, nullptr, cs, nullptr);
+        int rc = copy_chunk_out(h, G, p0, np, E, nullptr, cs, nullptr, c_bytes);
         if (rc) return rc;
         if (C)
             for (int p = p0; p < p0 + np; ++p) {
                 const long long nel = (long long)G.n * std::min(nsel[p - p0], G.nvec[p]);
                 if (nel > 0) {
                     CU(cudaMemcpyAsync(C + h->c_off[G.prob_index[p]], G.d_C + G.coff[p], sizeof(double) * (size_t)nel, cudaMemcpyDefault, cs));
-                    h->c_bytes_copied += 8 * nel;
+                    c_bytes += 8 * nel;
                 }
             }
         return 0;
     }
+    /* pencils of a group are usually contiguous in the caller's order: merge runs */
     int p = p0;
     while (p < p0 + np) {
         int q = p;
@@ -1012,7 +1015,7 @@ int copy_chunk_out(bspatom_handle h, Group &G, int p0, int np, double *E, double
             const long long nel = (q + 1 < G.npencil ? G.coff[q + 1] : G.c_elems) - G.coff[p];
             if (nel > 0) CU(cudaMemcpyAsync(C + h->c_off[i0], G.d_C + G.coff[p], sizeof(double) * (size_t)nel,
                                             cudaMemcpyDefault, cs));
-            h->c_bytes_copied += 8 * nel;
+            c_bytes += 8 * nel;
         }
         p = q + 1;
     }
@@ -1032,28 +1035,14 @@ extern "C" int bspatom_batch_run(bspatom_handle h)
 
 namespace {
 
-template <int B>
-int launch_pdcheck_b(bspatom_handle h, Group &G, cudaStream_t st)
-{
-    bsp_pdcheck_fast_kernel<B><<<(G.ninst + 31) / 32, 32, 0, st>>>(G.d_fbS, G.n, G.npad, G.nrows, G.ninst, G.d_pdinfo);
-    h->launches++;
-    CU(cudaGetLastError());
-    return 0;
-}
-
 int launch_pdcheck(bspatom_handle h, Group &G, cudaStream_t st)
 {
-    switch (G.B) {
-    case 2: return launch_pdcheck_b<2>(h, G, st);
-    case 3: return launch_pdcheck_b<3>(h, G, st);
-    case 4: return launch_pdcheck_b<4>(h, G, st);
-    case 5: return launch_pdcheck_b<5>(h, G, st);
-    case 6: return launch_pdcheck_b<6>(h, G, st);
-    case 7: return launch_pdcheck_b<7>(h, G, st);
-    case 8: return launch_pdcheck_b<8>(h, G, st);
-    case 9: return launch_pdcheck_b<9>(h, G, st);
-    default: return BSPATOM_EUNSUPPORTED;
-    }
+    return with_half_band(G.B, [&](auto B) {
+        bsp_pdcheck_fast_kernel<B><<<(G.ninst + 31) / 32, 32, 0, st>>>(G.d_fbS, G.n, G.npad, G.nrows, G.ninst, G.d_pdinfo);
+        h->launches++;
+        CU(cudaGetLastError());
+        return 0;
+    });
 }
 
 /* S, H0 and Q rows of every instance of an assembled group */
@@ -1075,17 +1064,125 @@ BspRunStats stats_from_report(const int *r)
     return st;
 }
 
-/* enqueue (on the copy stream, after the chunk's own stream reached this point) the D2H of a chunk */
-int stream_chunk_out(bspatom_handle h, bspatom_handle ctx, Group &G, int p0, int np, double *E_out, double *C_out,
-                     cudaStream_t cs)
+/* where a run streams its results: the caller's pinned E / C, through the device's copy queue */
+struct Delivery {
+    double *E, *C;
+    CopyQueue *cq;             /* null when nothing streams */
+    cudaEvent_t copies_done;   /* recorded behind the run's last copy */
+};
+
+/* enqueue on the copy stream, once the chunk is final, the D2H of its results (the selected columns with a
+ * device-side selection, whose counts must be in the mailbox by now); the caller holds the queue's lock */
+int copy_chunk(bspatom_handle h, Group &G, const ChunkRec &r, const Delivery &out)
 {
-    cudaEvent_t e;
-    CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    h->chunk_done.push_back(e);
-    CU(cudaEventRecord(e, ctx->st));
-    CU(cudaStreamWaitEvent(cs, e, 0));
-    return copy_chunk_out(h, G, p0, np, E_out, C_out, cs);
+    CU(cudaStreamWaitEvent(out.cq->st, r.done, 0));
+    if (r.c0) CU(cudaEventRecord(r.c0, out.cq->st));
+    long long bytes = 0;
+    const int rc = copy_chunk_out(h, G, r.p0, r.np, out.E, out.C, out.cq->st, G.any_sel ? h->h_sel + G.sel_off + r.p0 : nullptr, bytes);
+    if (rc) return rc;
+    h->c_bytes_copied += bytes;
+    if (r.c1) CU(cudaEventRecord(r.c1, out.cq->st));
+    return 0;
 }
+
+int copy_chunk_locked(bspatom_handle h, Group &G, const ChunkRec &r, const Delivery &out)
+{
+    std::lock_guard<std::mutex> lk(out.cq->mu);
+    const int rc = copy_chunk(h, G, r, out);
+    if (rc) return rc;
+    CU(cudaEventRecord(out.copies_done, out.cq->st));
+    return 0;
+}
+
+/* the control blocks of chunks [c0, c0 + count) into report: from the mailbox, or from the device */
+int read_reports(bspatom_handle h, const int *d_report, int c0, int count, int *report)
+{
+    const size_t off = (size_t)c0 * BSP_C_WORDS, bytes = (size_t)count * BSP_C_WORDS * sizeof(int);
+    if (d_report == h->h_counter_dev) memcpy(report + off, h->h_counter + off, bytes);
+    else CU(cudaMemcpy(report + off, d_report + off, bytes, cudaMemcpyDeviceToHost));
+    return 0;
+}
+
+/* chunk ci ran out of rounds or iterations: run it again with the full limits on h's own stream, copy its results
+ * again and re-read its report */
+int redo_chunk(bspatom_handle h, Group &G, int largest, ChunkRec &r, const BspSchedule &sch, int *d_report, int ci,
+               const Delivery &out, int *report)
+{
+    int rc;
+    ChunkPtrs cc;
+    carve_chunk(G, largest, h->ws.base, cc, use_ckpt(h, G));
+    CU(cudaMemsetAsync(G.d_bad + r.p0, 0, sizeof(int) * r.np, h->st));
+    if ((rc = enqueue_chunk(h, G, r.p0, r.np, cc, sch, r, d_report + (size_t)ci * BSP_C_WORDS))) return rc;
+    if (out.cq && !G.any_sel) {
+        CU(cudaEventRecord(r.done, h->st));
+        if ((rc = copy_chunk_locked(h, G, r, out))) return rc;
+    }
+    CU(cudaStreamSynchronize(h->st));
+    if (out.cq && G.any_sel && (rc = copy_chunk_locked(h, G, r, out))) return rc;   /* sized by the new counts */
+    return read_reports(h, d_report, ci, 1, report);
+}
+
+/* info flags of every group -> mailbox, on h's stream (all chunk streams are drained at this point) */
+int mail_info_flags(bspatom_handle h)
+{
+    size_t need = 0;
+    for (auto &G : h->groups) need += (size_t)G.ninst + (size_t)G.npencil;
+    h->mail_info = need <= (size_t)(BSP_MAIL_INTS - BSP_MAIL_REPORT_INTS);
+    if (!h->mail_info) return 0;
+    size_t off = BSP_MAIL_REPORT_INTS;
+    for (auto &G : h->groups) {
+        bsp_copy_ints_kernel<<<(G.ninst + 255) / 256, 256, 0, h->st>>>(h->h_counter_dev + off, G.d_pdinfo, G.ninst);
+        off += (size_t)G.ninst;
+        bsp_copy_ints_kernel<<<(G.npencil + 255) / 256, 256, 0, h->st>>>(h->h_counter_dev + off, G.d_bad, G.npencil);
+        off += (size_t)G.npencil;
+        h->launches += 2;
+    }
+    CU(cudaGetLastError());
+    return 0;
+}
+
+/* `workers` chunk streams with a workspace of `need` bytes each: h and helper contexts, which wait for `after` */
+int ready_streams(bspatom_handle h, int workers, size_t need, cudaEvent_t after, std::vector<bspatom_handle> &ctx)
+{
+    int rc;
+    if ((rc = ensure_workspace(h, need))) return rc;
+    while ((int)h->aux.size() < workers - 1) {
+        bspatom_handle x = new_context(h->dev);
+        if (!x) { h->err = "cannot create a helper chunk stream"; return BSPATOM_ECUDA; }
+        h->aux.push_back(x);
+    }
+    ctx.assign(1, h);
+    for (int w = 1; w < workers; ++w) {
+        h->aux[w - 1]->opt = h->opt;
+        if ((rc = ensure_workspace(h->aux[w - 1], need, h))) { h->err = h->aux[w - 1]->err; return rc; }
+        CU(cudaStreamWaitEvent(h->aux[w - 1]->st, after, 0));
+        ctx.push_back(h->aux[w - 1]);
+    }
+    return 0;
+}
+
+/* diagnostics (option trace): when each chunk was final and when its copy ran, in ms after e0 */
+void print_trace(bspatom_handle h, cudaEvent_t e0, const std::vector<ChunkRec> &recs)
+{
+    for (size_t ci = 0; ci < recs.size(); ++ci) {
+        float a = 0, b = 0, c = 0;
+        cudaEventElapsedTime(&a, e0, recs[ci].done); cudaEventElapsedTime(&b, e0, recs[ci].c0); cudaEventElapsedTime(&c, e0, recs[ci].c1);
+        fprintf(stderr, "[bspatom trace %p] chunk %d stream %d pencils %d final at %.2f ms, copy %.2f -> %.2f ms\n", (void *)h,
+                (int)ci, recs[ci].w, recs[ci].np, a, b, c);
+    }
+}
+
+/* events of a run, released on every exit (there are many CU(...) returns in run_internal) */
+struct EventGuard {
+    std::vector<cudaEvent_t> ev;
+    cudaEvent_t make(unsigned flags, cudaError_t &err) {
+        cudaEvent_t e = nullptr;
+        err = cudaEventCreateWithFlags(&e, flags);
+        if (err == cudaSuccess) ev.push_back(e);
+        return e;
+    }
+    ~EventGuard() { for (auto e : ev) cudaEventDestroy(e); }
+};
 
 /* E_out / C_out: pinned host buffers (or NULL).  Every chunk's whole schedule is enqueued up front on one
  * of `workers` streams (each with its own workspace) -- the host reads nothing back while the batch runs,
@@ -1112,17 +1209,7 @@ int run_internal(bspatom_handle h, double *E_out, double *C_out)
     int rounds = 0, iters = 0, redone = 0;
     long long selected = 0;
     h->c_bytes_copied = 0;
-    /* every exit (there are many CU(...) returns below) releases the events of the run */
-    struct EventGuard {
-        std::vector<cudaEvent_t> ev;
-        cudaEvent_t make(unsigned flags, cudaError_t &err) {
-            cudaEvent_t e = nullptr;
-            err = cudaEventCreateWithFlags(&e, flags);
-            if (err == cudaSuccess) ev.push_back(e);
-            return e;
-        }
-        ~EventGuard() { for (auto e : ev) cudaEventDestroy(e); }
-    } events;
+    EventGuard events;
     cudaError_t ev_err = cudaSuccess;
     cudaEvent_t e0 = events.make(cudaEventDefault, ev_err); CU(ev_err);
     cudaEvent_t e1 = events.make(cudaEventDefault, ev_err); CU(ev_err);
@@ -1130,11 +1217,12 @@ int run_internal(bspatom_handle h, double *E_out, double *C_out)
     cudaEvent_t copies_done = events.make(cudaEventDisableTiming, ev_err); CU(ev_err);
     cudaEvent_t pd_done = events.make(cudaEventDisableTiming, ev_err); CU(ev_err);
     CU(cudaEventRecord(pd_done, h->st_copy));
-    CopyQueue *cq = (E_out || C_out) ? copy_queue(h->dev) : nullptr;
-    if ((E_out || C_out) && !cq) { h->err = "cannot create the result-copy stream"; return BSPATOM_ECUDA; }
+    const bool streaming = (E_out || C_out);
+    const Delivery out = {E_out, C_out, streaming ? copy_queue(h->dev) : nullptr, copies_done};
+    if (streaming && !out.cq) { h->err = "cannot create the result-copy stream"; return BSPATOM_ECUDA; }
     std::unique_lock<std::mutex> turn;
-    if (cq) turn = std::unique_lock<std::mutex>(cq->turn);
-    if (cq) CU(cudaEventRecord(copies_done, cq->st));
+    if (streaming) turn = std::unique_lock<std::mutex>(out.cq->turn);
+    if (streaming) CU(cudaEventRecord(copies_done, out.cq->st));
     CU(cudaEventRecord(e0, h->st));
     const BspSchedule sch_vec = {std::min(h->opt.rounds_enqueued, h->opt.max_rounds), h->opt.min_iters,
                                  std::min(h->opt.max_iters, h->opt.min_iters + 3)};
@@ -1161,23 +1249,9 @@ int run_internal(bspatom_handle h, double *E_out, double *C_out)
         CU(cudaStreamWaitEvent(h->st_copy, e2, 0));
         if ((rc = launch_pdcheck(h, G, h->st_copy))) return rc;
         CU(cudaEventRecord(pd_done, h->st_copy));
-        /* ---- chunking ---- */
+        /* ---- chunking (bsp_plan.h) ---- */
         ChunkPtrs c;
         const size_t per_pencil = carve_chunk(G, 1, nullptr, c, use_ckpt(h, G));
-        const int blocks_per_pencil = (G.n + BSP_EIG_THREADS - 1) / BSP_EIG_THREADS;
-        const int fill_pencils = std::max(1, (148 * 4 + blocks_per_pencil - 1) / blocks_per_pencil); /* one full wave */
-        const bool streaming = (E_out || C_out);
-        /* Chunk streams: `workers` streams (each with its own workspace) run chunks concurrently and
-         * back-fill each other's partial waves and latency-bound kernels (late bracketing rounds); blocks
-         * run a whole sweep (~1 ms), so stream priorities cannot order the chunks -- the chunk sizes do.
-         * Resident batches use `workers` equal chunks.  When results stream to the host the D2H (PCIe,
-         * ~53 GB/s, 57 ms per 408 solves of N = 1000) is the longer leg: the batch is cut into
-         * `stream_chunks` chunks whose sizes SHRINK (weights n+2, n+1, ..., 3): the first copies start as
-         * early as with equal chunks and keep the link busy, and the last chunks -- whose copies nothing can
-         * hide -- are small.  (Measured, single handle, 408 solves: shrinking 79.6 ms, equal 84 ms, growing
-         * 95 ms per batch: a chunk below ~40 pencils takes ~17 ms whatever its size, its kernel chain being
-         * latency-bound, so small chunks must not come first.) */
-        int workers = std::max(1, std::min(streaming ? h->opt.stream_workers : h->opt.workers, G.npencil / fill_pencils));
         if (h->budget_bytes == 0) {
             /* once per handle: cudaMemGetInfo takes milliseconds and stalls behind whatever else the device is
              * doing (another handle's batch), which would delay every submission */
@@ -1188,74 +1262,18 @@ int run_internal(bspatom_handle h, double *E_out, double *C_out)
             h->budget_bytes = std::max<size_t>(std::min<size_t>((free_b + have) / 2, (size_t)64 << 30), 1);
         }
         G.budget_pencils = (int)std::max<size_t>(1, std::min<size_t>(h->budget_bytes / per_pencil, 1 << 24));
-        const int cap = std::max(1, std::min(G.budget_pencils / workers, 1024));   /* workspace per stream */
-        int chunk = h->opt.chunk, nchunks;
-        std::vector<int> bounds(1, 0);
-        if (chunk > 0) {
-            chunk = std::min(chunk, G.npencil);
-            nchunks = (G.npencil + chunk - 1) / chunk;
-            for (int i = 1; i <= nchunks; ++i) bounds.push_back(std::min(i * chunk, G.npencil));
-        } else {
-            int want = workers;
-            /* with a device-side selection the copies are small and every chunk carries the latency-bound tail of the
-             * rounds that close the values-only brackets: no extra chunks for streaming */
-            if (streaming && !G.any_sel) want = std::max(want, std::min(h->opt.stream_chunks, std::max(1, (2 * G.npencil) / fill_pencils)));
-            nchunks = std::max(want, (G.npencil + cap - 1) / cap);
-            nchunks = std::min(nchunks, G.npencil);
-            const bool shrink = streaming && nchunks >= 4 && (long long)cap * (nchunks + 5) >= 2LL * G.npencil;
-            if (shrink) {
-                /* weights n+2, n+1, ..., 3: the largest chunk is < 2x the mean and must fit the workspace */
-                double tot = 0.0, accw = 0.0;
-                for (int i = 0; i < nchunks; ++i) tot += (double)(nchunks + 2 - i);
-                for (int i = 0; i < nchunks; ++i) {
-                    accw += (double)(nchunks + 2 - i);
-                    int bnd = (i + 1 == nchunks) ? G.npencil : (int)(G.npencil * accw / tot + 0.5);
-                    bnd = std::max(bnd, bounds.back() + 1);
-                    bnd = std::min(bnd, G.npencil - (nchunks - 1 - i));
-                    bounds.push_back(bnd);
-                }
-            } else {
-                const int eq = (G.npencil + nchunks - 1) / nchunks;
-                nchunks = (G.npencil + eq - 1) / eq;
-                for (int i = 1; i <= nchunks; ++i) bounds.push_back(std::min(i * eq, G.npencil));
-            }
-            chunk = 0;
-            for (int i = 0; i < nchunks; ++i) chunk = std::max(chunk, bounds[i + 1] - bounds[i]);
+        BspPlanInput in;
+        in.npencil = G.npencil; in.n = G.n; in.budget_pencils = G.budget_pencils; in.streaming = streaming; in.chunk = h->opt.chunk;
+        in.workers = h->opt.workers; in.stream_workers = h->opt.stream_workers; in.stream_chunks = h->opt.stream_chunks;
+        if (G.any_sel) for (auto &sl : G.sel) in.sel.push_back({sl.mode, sl.group});
+        const BspChunkPlan plan = bsp_plan_chunks(in);
+        if (plan.group_too_large) {
+            h->err = "a selection group (sel_group) has more pencils than fit one chunk of the workspace";
+            return BSPATOM_ENOMEM;
         }
-        if (G.any_sel) {
-            /* the running maximum of a selection group is sequential over its pencils: a group stays in one chunk */
-            for (size_t b = 1; b + 1 < bounds.size(); ++b) {
-                int x = std::max(bounds[b], bounds[b - 1]);
-                while (x < G.npencil && x > 0 && G.sel[x].mode && G.sel[x].group >= 0 && G.sel[x - 1].mode &&
-                       G.sel[x - 1].group == G.sel[x].group) ++x;
-                bounds[b] = x;
-            }
-            std::vector<int> nb(1, 0);
-            for (size_t b = 1; b < bounds.size(); ++b) if (bounds[b] > nb.back()) nb.push_back(bounds[b]);
-            bounds = nb;
-            nchunks = (int)bounds.size() - 1;
-            chunk = 0;
-            for (int i = 0; i < nchunks; ++i) chunk = std::max(chunk, bounds[i + 1] - bounds[i]);
-            if (chunk > std::max(cap, 1) && h->opt.chunk <= 0) {
-                h->err = "a selection group (sel_group) has more pencils than fit one chunk of the workspace";
-                return BSPATOM_ENOMEM;
-            }
-        }
-        workers = std::min(workers, nchunks);
-        const size_t need = carve_chunk(G, chunk, nullptr, c, use_ckpt(h, G));
-        if ((rc = ensure_workspace(h, need))) return rc;
-        while ((int)h->aux.size() < workers - 1) {
-            bspatom_handle x = new_context(h->dev);
-            if (!x) { h->err = "cannot create a helper chunk stream"; return BSPATOM_ECUDA; }
-            h->aux.push_back(x);
-        }
-        std::vector<bspatom_handle> ctx(1, h);
-        for (int w = 1; w < workers; ++w) {
-            h->aux[w - 1]->opt = h->opt;
-            if ((rc = ensure_workspace(h->aux[w - 1], need, h))) { h->err = h->aux[w - 1]->err; return rc; }
-            CU(cudaStreamWaitEvent(h->aux[w - 1]->st, e2, 0));     /* after the assembly */
-            ctx.push_back(h->aux[w - 1]);
-        }
+        const int nchunks = plan.nchunks(), workers = plan.streams;
+        std::vector<bspatom_handle> ctx;   /* the chunk streams' contexts; helpers start after the assembly */
+        if ((rc = ready_streams(h, workers, carve_chunk(G, plan.largest, nullptr, c, use_ckpt(h, G)), e2, ctx))) return rc;
         /* ---- enqueue every chunk; no host read-back in here ---- */
         const bool report_mail = (size_t)nchunks * BSP_C_WORDS <= BSP_MAIL_REPORT_INTS;
         int *d_report = nullptr;
@@ -1268,157 +1286,99 @@ int run_internal(bspatom_handle h, double *E_out, double *C_out)
             if ((rc = dev_alloc(h, &d_report, (size_t)nchunks * BSP_C_WORDS))) return rc;
             report_guard.p = d_report; report_guard.count = (size_t)nchunks * BSP_C_WORDS;
         }
-        std::vector<ChunkTimes> tms(nchunks);
+        std::vector<ChunkRec> recs(nchunks);
         for (int ci = 0; ci < nchunks; ++ci) {
-            for (int i = 0; i < 4; ++i) { tms[ci].ev[i] = events.make(cudaEventDefault, ev_err); CU(ev_err); }
+            ChunkRec &r = recs[ci];
+            r.p0 = plan.bounds[ci]; r.np = plan.bounds[ci + 1] - r.p0;
+            for (int i = 0; i < 4; ++i) { r.ev[i] = events.make(cudaEventDefault, ev_err); CU(ev_err); }
             if (G.any_sel) {
-                tms[ci].selected = events.make(cudaEventDisableTiming, ev_err); CU(ev_err);
-                tms[ci].sel_report = h->h_sel_dev + G.sel_off + bounds[ci];
+                r.selected = events.make(cudaEventDisableTiming, ev_err); CU(ev_err);
+                r.sel_report = h->h_sel_dev + G.sel_off + r.p0;
+            }
+            if (streaming && h->opt.trace) {   /* diagnostics: when was the chunk final, when did its copy run */
+                r.c0 = events.make(cudaEventDefault, ev_err); CU(ev_err);
+                r.c1 = events.make(cudaEventDefault, ev_err); CU(ev_err);
             }
         }
-        std::vector<cudaEvent_t> final_ev(nchunks, nullptr);   /* selection mode: chunk final, copies not yet enqueued */
-        std::vector<bspatom_handle> chunk_ctx(nchunks, nullptr);
-        struct TraceRec { int ci, w, np; cudaEvent_t done, c0, c1; };
-        std::vector<TraceRec> trace;
         std::vector<long long> load(workers, 0);      /* pencils assigned to each stream so far */
         std::unique_lock<std::mutex> copy_lock;
         const double t_lock0 = host_ms();
-        if (streaming) copy_lock = std::unique_lock<std::mutex>(cq->mu);
+        if (streaming) copy_lock = std::unique_lock<std::mutex>(out.cq->mu);
         const double t_lock1 = host_ms();
         for (int ci = 0; ci < nchunks; ++ci) {
-            int wsel = 0;
-            for (int w = 1; w < workers; ++w) if (load[w] < load[wsel]) wsel = w;
-            load[wsel] += bounds[ci + 1] - bounds[ci];
-            bspatom_handle x = ctx[wsel];
+            ChunkRec &r = recs[ci];
+            for (int w = 1; w < workers; ++w) if (load[w] < load[r.w]) r.w = w;
+            load[r.w] += r.np;
+            bspatom_handle x = ctx[r.w];
             ChunkPtrs cc;
-            carve_chunk(G, chunk, x->ws.base, cc, use_ckpt(h, G));
-            const int p0 = bounds[ci], np = bounds[ci + 1] - p0;
-            if ((rc = enqueue_chunk(x, G, p0, np, cc, sch, tms[ci], d_report + (size_t)ci * BSP_C_WORDS))) {
+            carve_chunk(G, plan.largest, x->ws.base, cc, use_ckpt(h, G));
+            if ((rc = enqueue_chunk(x, G, r.p0, r.np, cc, sch, r, d_report + (size_t)ci * BSP_C_WORDS))) {
                 if (x != h) h->err = x->err;
                 return rc;
             }
-            chunk_ctx[ci] = x;
-            if ((E_out || C_out) && G.any_sel) {
-                /* the copies are sized by the selection: enqueued below, once the chunk's counts are in the mailbox */
-                CU(cudaEventCreateWithFlags(&final_ev[ci], cudaEventDisableTiming));
-                CU(cudaEventRecord(final_ev[ci], x->st));
-            } else if (E_out || C_out) {
-                if (h->opt.trace) {     /* diagnostics: when was the chunk final, when did its copy run */
-                    TraceRec tr = {ci, wsel, np, nullptr, nullptr, nullptr};
-                    CU(cudaEventCreate(&tr.done)); CU(cudaEventCreate(&tr.c0)); CU(cudaEventCreate(&tr.c1));
-                    CU(cudaEventRecord(tr.done, x->st));
-                    CU(cudaStreamWaitEvent(cq->st, tr.done, 0));
-                    CU(cudaEventRecord(tr.c0, cq->st));
-                    if ((rc = copy_chunk_out(h, G, p0, np, E_out, C_out, cq->st))) return rc;
-                    CU(cudaEventRecord(tr.c1, cq->st));
-                    trace.push_back(tr);
-                } else if ((rc = stream_chunk_out(h, x, G, p0, np, E_out, C_out, cq->st))) return rc;
-            }
+            if (!streaming) continue;
+            CU(cudaEventCreateWithFlags(&r.done, h->opt.trace ? cudaEventDefault : cudaEventDisableTiming));
+            h->chunk_done.push_back(r.done);
+            CU(cudaEventRecord(r.done, x->st));
+            /* copies sized by a device-side selection are enqueued below, once the chunk's counts are in the mailbox */
+            if (!G.any_sel && (rc = copy_chunk(h, G, r, out))) return rc;
         }
-        if (streaming && G.any_sel) {
-            for (int ci = 0; ci < nchunks; ++ci) {
+        if (streaming && G.any_sel)
+            for (auto &r : recs) {
                 /* the selection kernel of the chunk ran right after its bracketing: its counts are in the mapped
                  * mailbox long before the vectors are final */
-                CU(cudaEventSynchronize(tms[ci].selected));
-                CU(cudaStreamWaitEvent(cq->st, final_ev[ci], 0));
-                h->chunk_done.push_back(final_ev[ci]);
-                if ((rc = copy_chunk_out(h, G, bounds[ci], bounds[ci + 1] - bounds[ci], E_out, C_out, cq->st,
-                                         h->h_sel + G.sel_off + bounds[ci]))) return rc;
+                CU(cudaEventSynchronize(r.selected));
+                if ((rc = copy_chunk(h, G, r, out))) return rc;
             }
-        }
         if (streaming) {
-            CU(cudaEventRecord(copies_done, cq->st));   /* behind this batch's last copy */
+            CU(cudaEventRecord(copies_done, out.cq->st));   /* behind this batch's last copy */
             copy_lock.unlock();
         }
         const double t_enq = host_ms();
         if (streaming && &G == &h->groups.back()) {
             /* pass the compute turn on once only the last (small) chunks are left */
-            const int k = nchunks >= 4 ? nchunks - 3 : nchunks - 1;
-            cudaEvent_t ev = trace.empty() ? h->chunk_done[h->chunk_done.size() - (size_t)nchunks + (size_t)k] : trace[(size_t)k].done;
-            CU(cudaEventSynchronize(ev));
+            CU(cudaEventSynchronize(recs[nchunks >= 4 ? nchunks - 3 : nchunks - 1].done));
             turn.unlock();
         }
         for (auto x : ctx) CU(cudaStreamSynchronize(x->st));
         if (h->opt.trace)
             fprintf(stderr, "[bspatom trace %p] host clock %.1f ms: entered run; +%.1f lock wait %.1f; +%.1f enqueued; +%.1f kernels done\n",
                     (void *)h, t_run0, t_lock0 - t_run0, t_lock1 - t_lock0, t_enq - t_run0, host_ms() - t_run0);
-        if (!trace.empty()) {
+        if (streaming && h->opt.trace) {
             CU(cudaEventSynchronize(copies_done));
-            for (auto &tr : trace) {
-                float a = 0, b = 0, c = 0;
-                cudaEventElapsedTime(&a, e0, tr.done); cudaEventElapsedTime(&b, e0, tr.c0); cudaEventElapsedTime(&c, e0, tr.c1);
-                fprintf(stderr, "[bspatom trace %p] chunk %d stream %d pencils %d final at %.2f ms, copy %.2f -> %.2f ms\n", (void *)h,
-                        tr.ci, tr.w, tr.np, a, b, c);
-                cudaEventDestroy(tr.done); cudaEventDestroy(tr.c0); cudaEventDestroy(tr.c1);
-            }
-            trace.clear();
+            print_trace(h, e0, recs);
         }
         /* ---- reports; chunks that ran out of rounds / iterations are redone with the full limits ---- */
         std::vector<int> report((size_t)nchunks * BSP_C_WORDS);
-        if (report_mail) memcpy(report.data(), h->h_counter, report.size() * sizeof(int));
-        else CU(cudaMemcpy(report.data(), d_report, report.size() * sizeof(int), cudaMemcpyDeviceToHost));
+        if ((rc = read_reports(h, d_report, 0, nchunks, report.data()))) return rc;
         for (int ci = 0; ci < nchunks; ++ci) {
             BspRunStats st = stats_from_report(&report[(size_t)ci * BSP_C_WORDS]);
             const bool again = (st.brackets_crowded > 0 || st.unconverged > 0) &&
                                (sch.rounds < sch_redo.rounds || sch.max_iters < sch_redo.max_iters);
             if (again) {
                 ++redone;
-                ChunkPtrs cc;
-                carve_chunk(G, chunk, h->ws.base, cc, use_ckpt(h, G));
-                const int p0 = bounds[ci], np = bounds[ci + 1] - p0;
-                CU(cudaMemsetAsync(G.d_bad + p0, 0, sizeof(int) * np, h->st));
-                if ((rc = enqueue_chunk(h, G, p0, np, cc, sch_redo, tms[ci], d_report + (size_t)ci * BSP_C_WORDS))) return rc;
-                if (streaming && !G.any_sel) {
-                    std::lock_guard<std::mutex> lk(cq->mu);
-                    if ((rc = stream_chunk_out(h, h, G, p0, np, E_out, C_out, cq->st))) return rc;
-                    CU(cudaEventRecord(copies_done, cq->st));
-                }
-                CU(cudaStreamSynchronize(h->st));
-                if (streaming && G.any_sel) {      /* the redone chunk's counts are in the mailbox now */
-                    std::lock_guard<std::mutex> lk(cq->mu);
-                    if ((rc = copy_chunk_out(h, G, p0, np, E_out, C_out, cq->st, h->h_sel + G.sel_off + p0))) return rc;
-                    CU(cudaEventRecord(copies_done, cq->st));
-                }
-                if (report_mail) memcpy(&report[(size_t)ci * BSP_C_WORDS], h->h_counter + (size_t)ci * BSP_C_WORDS, BSP_C_WORDS * sizeof(int));
-                else CU(cudaMemcpy(&report[(size_t)ci * BSP_C_WORDS], d_report + (size_t)ci * BSP_C_WORDS, BSP_C_WORDS * sizeof(int),
-                                   cudaMemcpyDeviceToHost));
+                if ((rc = redo_chunk(h, G, plan.largest, recs[ci], sch_redo, d_report, ci, out, report.data()))) return rc;
                 st = stats_from_report(&report[(size_t)ci * BSP_C_WORDS]);
             }
             rounds = std::max(rounds, st.rounds);
             iters = std::max(iters, st.iters);
             selected += report[(size_t)ci * BSP_C_WORDS + BSP_C_SELECTED];
             float ms = 0;
-            CU(cudaEventElapsedTime(&ms, tms[ci].ev[0], tms[ci].ev[1])); t_val += ms;
-            CU(cudaEventElapsedTime(&ms, tms[ci].ev[1], tms[ci].ev[2])); t_vec += ms;
-            CU(cudaEventElapsedTime(&ms, tms[ci].ev[2], tms[ci].ev[3])); t_fin += ms;
+            CU(cudaEventElapsedTime(&ms, recs[ci].ev[0], recs[ci].ev[1])); t_val += ms;
+            CU(cudaEventElapsedTime(&ms, recs[ci].ev[1], recs[ci].ev[2])); t_vec += ms;
+            CU(cudaEventElapsedTime(&ms, recs[ci].ev[2], recs[ci].ev[3])); t_fin += ms;
         }
         for (auto x : ctx) timed_collect(x);
         float ms = 0;
         CU(cudaEventElapsedTime(&ms, e1, e2)); t_asm += ms;
     }
     CU(cudaStreamWaitEvent(h->st, pd_done, 0));
-    /* info flags of every group -> mailbox (all chunk streams are drained at this point) */
-    {
-        size_t need = 0;
-        for (auto &G : h->groups) need += (size_t)G.ninst + (size_t)G.npencil;
-        h->mail_info = need <= (size_t)(BSP_MAIL_INTS - BSP_MAIL_REPORT_INTS);
-        if (h->mail_info) {
-            size_t off = BSP_MAIL_REPORT_INTS;
-            for (auto &G : h->groups) {
-                bsp_copy_ints_kernel<<<(G.ninst + 255) / 256, 256, 0, h->st>>>(h->h_counter_dev + off, G.d_pdinfo, G.ninst);
-                off += (size_t)G.ninst;
-                bsp_copy_ints_kernel<<<(G.npencil + 255) / 256, 256, 0, h->st>>>(h->h_counter_dev + off, G.d_bad, G.npencil);
-                off += (size_t)G.npencil;
-                h->launches += 2;
-            }
-            CU(cudaGetLastError());
-        }
-    }
+    if ((rc = mail_info_flags(h))) return rc;
     CU(cudaEventRecord(e1, h->st));   /* every chunk stream has been drained */
     CU(cudaStreamSynchronize(h->st));
     {
         auto t0 = std::chrono::steady_clock::now();
-        if (E_out || C_out) CU(cudaEventSynchronize(copies_done));
+        if (streaming) CU(cudaEventSynchronize(copies_done));
         h->stats[21] = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
     }
     float total = 0;
@@ -1436,7 +1396,6 @@ int run_internal(bspatom_handle h, double *E_out, double *C_out)
     h->ran = true;
     return 0;
 }
-
 } // namespace
 
 extern "C" {
@@ -1461,26 +1420,9 @@ int bspatom_batch_download(bspatom_handle h, double *E, double *C, int *info)
             CU(cudaMemcpyAsync(G.pdinfo.data(), G.d_pdinfo, sizeof(int) * G.ninst, cudaMemcpyDeviceToHost, h->st));
             CU(cudaMemcpyAsync(G.bad.data(), G.d_bad, sizeof(int) * G.npencil, cudaMemcpyDeviceToHost, h->st));
         }
-        if (G.any_sel) {   /* selected columns only */
-            if ((rc = copy_chunk_out(h, G, 0, G.npencil, E, C, h->st, h->h_sel + G.sel_off))) return rc;
-            continue;
-        }
-        /* pencils of a group are usually contiguous in the caller's order: merge runs */
-        int p = 0;
-        while (p < G.npencil) {
-            int q = p;
-            while (q + 1 < G.npencil && G.prob_index[q + 1] == G.prob_index[q] + 1) ++q;
-            const int i0 = G.prob_index[p];
-            const int cnt = q - p + 1;
-            if (E) CU(cudaMemcpyAsync(E + h->e_off[i0], G.d_E + (size_t)p * G.n, sizeof(double) * (size_t)cnt * G.n,
-                                      cudaMemcpyDefault, h->st));
-            if (C) {
-                const long long nel = (q + 1 < G.npencil ? G.coff[q + 1] : G.c_elems) - G.coff[p];
-                if (nel > 0) CU(cudaMemcpyAsync(C + h->c_off[i0], G.d_C + G.coff[p], sizeof(double) * (size_t)nel,
-                                                cudaMemcpyDefault, h->st));
-            }
-            p = q + 1;
-        }
+        long long bytes = 0;
+        if ((rc = copy_chunk_out(h, G, 0, G.npencil, E, C, h->st, G.any_sel ? h->h_sel + G.sel_off : nullptr, bytes))) return rc;
+        if (G.any_sel) h->c_bytes_copied += bytes;   /* selected columns only */
     }
     CU(cudaStreamSynchronize(h->st));
     if (info) {
@@ -1631,12 +1573,8 @@ int bspatom_band_upload(bspatom_handle h, int nprob, const bsp_band_pencil *pens
             members.emplace_back();
             Group &G = h->groups.back();
             G.band = true;
-            G.k = B + 1; G.B = B; G.n = q.n; G.nkp = q.n + G.k; G.ka = 1;
-            G.FS = 2 * B + 2;
-            G.npad = BSP_NPAD(G.n, B);
-            G.nrows = BSP_NROWS(G.npad, B);
-            G.xrows = G.npad + B + 1;
-            G.ldw = ((G.n + 31) / 32) * 32;
+            G.k = B + 1; G.nkp = q.n + G.k; G.ka = 1;
+            set_geometry(G, q.n, B);
         }
         members[it->second].push_back(i);
         ++ndesc;
@@ -1679,11 +1617,7 @@ int bspatom_band_upload(bspatom_handle h, int nprob, const bsp_band_pencil *pens
     for (size_t gi = 0; gi < h->groups.size(); ++gi) {
         Group &G = h->groups[gi];
         G.ninst = (int)members[gi].size();
-        const size_t per_mat = (size_t)G.nrows * G.FS;
-        if ((rc = dev_alloc(h, &G.d_fbS, per_mat * G.ninst))) return rc;
-        if ((rc = dev_alloc(h, &G.d_fbH0, per_mat * G.ninst))) return rc;
-        if ((rc = dev_alloc(h, &G.d_fbQ, per_mat * G.ninst))) return rc;
-        if ((rc = dev_alloc(h, &G.d_pdinfo, G.ninst))) return rc;
+        if ((rc = alloc_group_rows(h, G))) return rc;
         const unsigned grid = (unsigned)((G.nrows + BSP_INGEST_TR - 1) / BSP_INGEST_TR) * (unsigned)G.ninst;
         bsp_band_ingest_kernel<<<grid, BSP_INGEST_THREADS, 0, h->st>>>(d_stage, (const BspBandSrc *)d_stage + d, G.n, G.B,
                                                                      G.nrows, G.d_fbS, G.d_fbH0, G.d_fbQ);
@@ -1738,9 +1672,8 @@ int bspatom_assemble_band(bspatom_handle h, const bsp_problem *p, double *S, dou
     q.l = 0; q.nvec = 0;
     if ((rc = validate_problem(q))) return rc;
     Group G;
-    G.k = q.k; G.B = q.k - 1; G.n = q.nfun; G.nkp = q.nkp; G.ka = q.ka; G.FS = 2 * G.B + 2;
-    G.npad = BSP_NPAD(G.n, G.B);
-    G.nrows = BSP_NROWS(G.npad, G.B);
+    G.k = q.k; G.nkp = q.nkp; G.ka = q.ka;
+    set_geometry(G, q.nfun, q.k - 1);
     std::vector<const bsp_problem *> insts = {&q};
     G.ninst = 1;
     if ((rc = upload_group_instances(h, G, insts))) { free_group(h, G); return rc; }
@@ -1827,23 +1760,6 @@ int enqueue_shifted_b(bspatom_handle h, const BspShiftChunk<T> &c, const long lo
     if (c.nrhs > 0) { bsp_shifted_layout_kernel<T, false><<<lay, lay_t, 0, h->st>>>(c, d_off, d_X, c.X, d_info_out); h->launches++; }
     CU(cudaGetLastError());
     return 0;
-}
-
-template <class T>
-int enqueue_shifted(bspatom_handle h, int B, const BspShiftChunk<T> &c, const long long *d_off, T *d_B, T *d_X, int *d_info_out,
-                    double *d_berr_out)
-{
-    switch (B) {
-    case 2: return enqueue_shifted_b<2, T>(h, c, d_off, d_B, d_X, d_info_out, d_berr_out);
-    case 3: return enqueue_shifted_b<3, T>(h, c, d_off, d_B, d_X, d_info_out, d_berr_out);
-    case 4: return enqueue_shifted_b<4, T>(h, c, d_off, d_B, d_X, d_info_out, d_berr_out);
-    case 5: return enqueue_shifted_b<5, T>(h, c, d_off, d_B, d_X, d_info_out, d_berr_out);
-    case 6: return enqueue_shifted_b<6, T>(h, c, d_off, d_B, d_X, d_info_out, d_berr_out);
-    case 7: return enqueue_shifted_b<7, T>(h, c, d_off, d_B, d_X, d_info_out, d_berr_out);
-    case 8: return enqueue_shifted_b<8, T>(h, c, d_off, d_B, d_X, d_info_out, d_berr_out);
-    case 9: return enqueue_shifted_b<9, T>(h, c, d_off, d_B, d_X, d_info_out, d_berr_out);
-    default: return BSPATOM_EUNSUPPORTED;
-    }
 }
 
 /* device bytes of a chunk: per slot (factor, x, Y, b, state) and per pencil (its H_l rows) */
@@ -2027,7 +1943,8 @@ int shifted_solve(bspatom_handle h, int nsys, const int *iprob, const double *z,
                 bsp_combine_kernel<<<grid, 256, 0, h->st>>>(d_fbH, G.d_fbH0, G.d_fbQ, d_pen_inst, d_cl, per_mat);
                 h->launches++;
             }
-            if ((rc = enqueue_shifted<T>(h, G.B, c, d_off, d_B, d_X, d_info_out, d_berr_out))) return rc;
+            rc = with_half_band(G.B, [&](auto B) { return enqueue_shifted_b<B, T>(h, c, d_off, d_B, d_X, d_info_out, d_berr_out); });
+            if (rc) return rc;
             CU(cudaEventRecord(ev1, h->st));
             std::vector<int> iout(nslot);
             std::vector<double> bout(nslot);

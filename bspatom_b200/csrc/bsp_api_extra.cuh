@@ -54,13 +54,27 @@ __global__ void bsp_wavefunction_kernel(int nfun, int nkp, const double *__restr
     }
 }
 
-template <int K>
-void launch_wavefunction(bspatom_handle h, int nfun, int nkp, const double *rt, double ra, double rb, int npts,
-                         int nvec, const double *C, double *r_out, double *psi)
+/* r and psi on npts + 1 points of the nvec vectors at C (B-splines of order k = 3..10 on the knots rt, all on the
+ * device) into the caller's r_out / psi_out */
+int wavefunction_out(bspatom_handle h, int k, int nfun, int nkp, const double *rt, double ra, double rb, int npts,
+                     int nvec, const double *C, double *r_out, double *psi_out)
 {
-    dim3 grid((npts + 1 + 127) / 128, std::min(nvec, 64));
-    bsp_wavefunction_kernel<K><<<grid, 128, 0, h->st>>>(nfun, nkp, rt, ra, rb, npts, nvec, C, r_out, psi);
+    int rc;
+    double *d_r = nullptr, *d_psi = nullptr;
+    if ((rc = dev_alloc(h, &d_r, (size_t)npts + 1))) return rc;
+    if ((rc = dev_alloc(h, &d_psi, (size_t)(npts + 1) * nvec))) return rc;
+    const dim3 grid((npts + 1 + 127) / 128, std::min(nvec, 64));
+    with_order(k, [&](auto K) {
+        bsp_wavefunction_kernel<K><<<grid, 128, 0, h->st>>>(nfun, nkp, rt, ra, rb, npts, nvec, C, d_r, d_psi);
+        return 0;
+    });
     h->launches++;
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(r_out, d_r, sizeof(double) * ((size_t)npts + 1), cudaMemcpyDeviceToHost, h->st));
+    CU(cudaMemcpyAsync(psi_out, d_psi, sizeof(double) * (size_t)(npts + 1) * nvec, cudaMemcpyDeviceToHost, h->st));
+    CU(cudaStreamSynchronize(h->st));
+    dev_free(h, d_r, (size_t)npts + 1); dev_free(h, d_psi, (size_t)(npts + 1) * nvec);
+    return 0;
 }
 
 /* ---- device-side verification of a resident batch (bspatom_batch_verify) --------------------------------- *
@@ -160,29 +174,13 @@ int bspatom_wavefunction(bspatom_handle h, int k, int nfun, int nkp, const doubl
     if (rc) return rc;
     if (k < BSP_KMIN || k > BSP_KMAX) return BSPATOM_EUNSUPPORTED;
     if (nfun < 1 || nkp != nfun + k || !rt || npts < 1 || nvec < 1 || !C || !r_out || !psi_out) return -2;
-    double *d_rt = nullptr, *d_C = nullptr, *d_r = nullptr, *d_psi = nullptr;
+    double *d_rt = nullptr, *d_C = nullptr;
     if ((rc = dev_alloc(h, &d_rt, (size_t)nkp))) return rc;
     if ((rc = dev_alloc(h, &d_C, (size_t)nfun * nvec))) return rc;
-    if ((rc = dev_alloc(h, &d_r, (size_t)npts + 1))) return rc;
-    if ((rc = dev_alloc(h, &d_psi, (size_t)(npts + 1) * nvec))) return rc;
     CU(cudaMemcpyAsync(d_rt, rt, sizeof(double) * nkp, cudaMemcpyHostToDevice, h->st));
     CU(cudaMemcpyAsync(d_C, C, sizeof(double) * (size_t)nfun * nvec, cudaMemcpyHostToDevice, h->st));
-    switch (k) {
-    case 3: launch_wavefunction<3>(h, nfun, nkp, d_rt, ra, rb, npts, nvec, d_C, d_r, d_psi); break;
-    case 4: launch_wavefunction<4>(h, nfun, nkp, d_rt, ra, rb, npts, nvec, d_C, d_r, d_psi); break;
-    case 5: launch_wavefunction<5>(h, nfun, nkp, d_rt, ra, rb, npts, nvec, d_C, d_r, d_psi); break;
-    case 6: launch_wavefunction<6>(h, nfun, nkp, d_rt, ra, rb, npts, nvec, d_C, d_r, d_psi); break;
-    case 7: launch_wavefunction<7>(h, nfun, nkp, d_rt, ra, rb, npts, nvec, d_C, d_r, d_psi); break;
-    case 8: launch_wavefunction<8>(h, nfun, nkp, d_rt, ra, rb, npts, nvec, d_C, d_r, d_psi); break;
-    case 9: launch_wavefunction<9>(h, nfun, nkp, d_rt, ra, rb, npts, nvec, d_C, d_r, d_psi); break;
-    default: launch_wavefunction<10>(h, nfun, nkp, d_rt, ra, rb, npts, nvec, d_C, d_r, d_psi); break;
-    }
-    CU(cudaGetLastError());
-    CU(cudaMemcpyAsync(r_out, d_r, sizeof(double) * ((size_t)npts + 1), cudaMemcpyDeviceToHost, h->st));
-    CU(cudaMemcpyAsync(psi_out, d_psi, sizeof(double) * (size_t)(npts + 1) * nvec, cudaMemcpyDeviceToHost, h->st));
-    CU(cudaStreamSynchronize(h->st));
+    if ((rc = wavefunction_out(h, k, nfun, nkp, d_rt, ra, rb, npts, nvec, d_C, r_out, psi_out))) return rc;
     dev_free(h, d_rt, (size_t)nkp); dev_free(h, d_C, (size_t)nfun * nvec);
-    dev_free(h, d_r, (size_t)npts + 1); dev_free(h, d_psi, (size_t)(npts + 1) * nvec);
     return 0;
 }
 
@@ -368,27 +366,8 @@ int bspatom_wavefunction_resident(bspatom_handle h, int iprob, int ivec0, int nv
     if (iprob < 0 || iprob >= h->nprob || !find_resident(h, iprob, G, p)) return -2;
     if (ivec0 < 0 || nvec < 1 || ivec0 + nvec > resident_nvec(h, *G, p)) return -3;
     if (npts < 1 || !r_out || !psi_out) return -6;
-    double *d_r = nullptr, *d_psi = nullptr;
-    if ((rc = dev_alloc(h, &d_r, (size_t)npts + 1))) return rc;
-    if ((rc = dev_alloc(h, &d_psi, (size_t)(npts + 1) * nvec))) return rc;
-    const double *d_rt = G->d_rt + (size_t)G->inst[p] * G->nkp;
-    const double *d_C = G->d_C + G->coff[p] + (size_t)ivec0 * G->n;
-    switch (G->k) {
-    case 3: launch_wavefunction<3>(h, G->n, G->nkp, d_rt, ra, rb, npts, nvec, d_C, d_r, d_psi); break;
-    case 4: launch_wavefunction<4>(h, G->n, G->nkp, d_rt, ra, rb, npts, nvec, d_C, d_r, d_psi); break;
-    case 5: launch_wavefunction<5>(h, G->n, G->nkp, d_rt, ra, rb, npts, nvec, d_C, d_r, d_psi); break;
-    case 6: launch_wavefunction<6>(h, G->n, G->nkp, d_rt, ra, rb, npts, nvec, d_C, d_r, d_psi); break;
-    case 7: launch_wavefunction<7>(h, G->n, G->nkp, d_rt, ra, rb, npts, nvec, d_C, d_r, d_psi); break;
-    case 8: launch_wavefunction<8>(h, G->n, G->nkp, d_rt, ra, rb, npts, nvec, d_C, d_r, d_psi); break;
-    case 9: launch_wavefunction<9>(h, G->n, G->nkp, d_rt, ra, rb, npts, nvec, d_C, d_r, d_psi); break;
-    default: launch_wavefunction<10>(h, G->n, G->nkp, d_rt, ra, rb, npts, nvec, d_C, d_r, d_psi); break;
-    }
-    CU(cudaGetLastError());
-    CU(cudaMemcpyAsync(r_out, d_r, sizeof(double) * ((size_t)npts + 1), cudaMemcpyDeviceToHost, h->st));
-    CU(cudaMemcpyAsync(psi_out, d_psi, sizeof(double) * (size_t)(npts + 1) * nvec, cudaMemcpyDeviceToHost, h->st));
-    CU(cudaStreamSynchronize(h->st));
-    dev_free(h, d_r, (size_t)npts + 1); dev_free(h, d_psi, (size_t)(npts + 1) * nvec);
-    return 0;
+    return wavefunction_out(h, G->k, G->n, G->nkp, G->d_rt + (size_t)G->inst[p] * G->nkp, ra, rb, npts, nvec,
+                            G->d_C + G->coff[p] + (size_t)ivec0 * G->n, r_out, psi_out);
 }
 
 /* General (structured-light) branch of TRANS_AMP, PhotoIon.f90:218-232: for one angular block (il, jl, component)
@@ -587,9 +566,8 @@ int bspatom_assemble_zaij(bspatom_handle h, const bsp_problem *p, int kind_pi, i
     }
     if (ncomp_in < need_in) return -5;
     Group G;
-    G.k = q.k; G.B = q.k - 1; G.n = q.nfun; G.nkp = q.nkp; G.ka = q.ka; G.FS = 2 * G.B + 2;
-    G.npad = BSP_NPAD(G.n, G.B);
-    G.nrows = BSP_NROWS(G.npad, G.B);
+    G.k = q.k; G.nkp = q.nkp; G.ka = q.ka;
+    set_geometry(G, q.nfun, q.k - 1);
     std::vector<const bsp_problem *> insts = {&q};
     G.ninst = 1;
     if ((rc = upload_group_instances(h, G, insts))) { free_group(h, G); return rc; }
@@ -609,14 +587,11 @@ int bspatom_assemble_zaij(bspatom_handle h, const bsp_problem *p, int kind_pi, i
     const dim3 grid((n + BSP_ZTR - 1) / BSP_ZTR, nblk);
     const size_t smem = sizeof(double) * (size_t)(BSP_ZTR + q.k - 1) * q.ka * (2 * q.k + 2);
     if (e == cudaSuccess) {
-        switch (q.k) {
-#define BSP_Z_CASE(K_) case K_: \
-            e = cudaFuncSetAttribute(bsp_assemble_zaij_kernel<K_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-            if (e == cudaSuccess) bsp_assemble_zaij_kernel<K_><<<grid, 128, smem, h->st>>>(a); break;
-            BSP_Z_CASE(3) BSP_Z_CASE(4) BSP_Z_CASE(5) BSP_Z_CASE(6) BSP_Z_CASE(7) BSP_Z_CASE(8) BSP_Z_CASE(9) BSP_Z_CASE(10)
-#undef BSP_Z_CASE
-        default: rc = BSPATOM_EUNSUPPORTED; break;
-        }
+        rc = with_order(q.k, [&](auto K) {
+            e = cudaFuncSetAttribute(bsp_assemble_zaij_kernel<K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+            if (e == cudaSuccess) bsp_assemble_zaij_kernel<K><<<grid, 128, smem, h->st>>>(a);
+            return 0;
+        });
         h->launches++;
     }
     if (e == cudaSuccess && !rc) e = cudaGetLastError();
@@ -737,9 +712,8 @@ void bspatom_dsygv_(const int *itype, const char *jobz, const char *uplo, const 
     if (kd > BSP_KMAX - 1) { *info = -5; h->err = "bspatom_dsygv_: pencil half bandwidth exceeds 9"; return; }
     const int B = std::max(kd, BSP_KMIN - 1);
     Group G;
-    G.k = B + 1; G.B = B; G.n = n; G.nkp = n + G.k; G.ka = 1; G.FS = 2 * B + 2;
-    G.npad = BSP_NPAD(n, B);
-    G.nrows = BSP_NROWS(G.npad, B); G.xrows = G.npad + B + 1; G.ldw = ((n + 31) / 32) * 32;
+    G.k = B + 1; G.nkp = n + G.k; G.ka = 1;
+    set_geometry(G, n, B);
     G.ninst = 1; G.npencil = 1;
     G.prob_index = {0}; G.inst = {0}; G.nvec = {wantz ? n : 0}; G.cl = {0.0}; G.coff = {0};
     G.c_elems = wantz ? (long long)n * n : 0;
@@ -759,14 +733,11 @@ void bspatom_dsygv_(const int *itype, const char *jobz, const char *uplo, const 
     int rc = 0;
     double *d_L = nullptr;
     do {
-        if ((rc = dev_alloc(h, &G.d_fbS, per_mat))) break;
-        if ((rc = dev_alloc(h, &G.d_fbH0, per_mat))) break;
-        if ((rc = dev_alloc(h, &G.d_fbQ, per_mat))) break;
+        if ((rc = alloc_group_rows(h, G))) break;
         if ((rc = dev_alloc(h, &G.d_inst, 1))) break;
         if ((rc = dev_alloc(h, &G.d_nvec, 1))) break;
         if ((rc = dev_alloc(h, &G.d_cl, 1))) break;
         if ((rc = dev_alloc(h, &G.d_coff, 1))) break;
-        if ((rc = dev_alloc(h, &G.d_pdinfo, 1))) break;
         if ((rc = dev_alloc(h, &G.d_bad, 1))) break;
         if ((rc = dev_alloc(h, &G.d_E, (size_t)n))) break;
         if ((rc = dev_alloc(h, &G.d_C, (size_t)G.c_elems))) break;
@@ -800,7 +771,7 @@ void bspatom_dsygv_(const int *itype, const char *jobz, const char *uplo, const 
     Group &GG = h->groups.back();
     ChunkPtrs c;
     const size_t need = carve_chunk(GG, 1, nullptr, c, use_ckpt(h, GG));
-    ChunkTimes tm;
+    ChunkRec tm;
     bool ev_ok = true;
     for (int i = 0; i < 4; ++i) ev_ok = ev_ok && (cudaEventCreate(&tm.ev[i]) == cudaSuccess);
     rc = ev_ok ? ensure_workspace(h, need) : BSPATOM_ECUDA;
